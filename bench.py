@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W              # this repo's CUDA path (one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU algorithm (oracle port)
+    python bench.py ... --dump-outputs DIR                     # also write the last timed step's Gram to DIR/gram.npy
 
 Workload (config.workload): BASELINE.json configs[1] -- 2504 samples x 1 M variants, int8 binary carrier encoding,
 per GPU (weak scaling: every rank owns `--variants-per-gpu` variants; 8 ranks x 5 M is configs[2]).  Synthetic
@@ -69,7 +70,12 @@ def parse_args():
     ap.add_argument("--c5-samples", type=int, default=10_000)
     ap.add_argument("--c5-variants-per-gpu", type=int, default=1_250_000, help="0 disables the c5_bf16 leg")
     ap.add_argument("--no-legs", action="store_true", help="skip the c3 and c5_bf16 legs (quick kernel A/B runs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the Gram of the last one to DIR/gram.npy (see dump_gram)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def load_peaks():
@@ -80,6 +86,28 @@ def load_peaks():
                 "bf16_tflops_sustained": float(d.get("bf16_tflops_sustained", 1400.0)),
                 "hbm_gbs": float(d.get("hbm_gbs", 6650.0)), "source": "measured"}
     return {"bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0, "hbm_gbs": 6650.0, "source": "fallback"}
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_gram(out_dir, S):
+    """--dump-outputs: the symmetrized N x N Gram a step hands its caller, as DIR/gram.npy in float64 (exact for every
+    int32 count), so that two builds run with the same arguments can be compared entry for entry.  A Gram larger than
+    DUMP_BYTES is sampled: whole rows drawn by a generator seeded with SEED (the same rows on every run), their indices
+    in DIR/gram_rows.npy."""
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    n = S.shape[0]
+    rows_file = out / "gram_rows.npy"
+    if 8 * S.size > DUMP_BYTES - 4096:                   # 4096: room for the .npy headers
+        rows = np.sort(np.random.default_rng(SEED).choice(n, size=(DUMP_BYTES - 4096) // (8 * (n + 1)), replace=False))
+        S = S[rows]
+        np.save(rows_file, rows.astype(np.float64))
+    else:
+        rows_file.unlink(missing_ok=True)
+    np.save(out / "gram.npy", S.astype(np.float64))
 
 
 class ClockSampler(threading.Thread):
@@ -188,7 +216,7 @@ def cpu_similarity_sample(n, variants=32768, threads=None, repeats=5):
     times = sorted(times[1:]) if len(times) > 1 else times
     med = times[len(times) // 2]
     return n * nv / med, {"variants": nv, "seconds": med, "seconds_all": [round(t, 4) for t in times], "threads": threads,
-                          "numa": numa_policy(), "checksum": int(S.trace())}
+                          "numa": numa_policy(), "checksum": int(S.trace()), "gram": S}
 
 
 def cpu_blas_sample(n, nv=65_536, threads=None):
@@ -249,6 +277,8 @@ def run_reference(args):
         v, info = cpu_similarity_sample(n, args.cpu_sample_variants, threads, repeats=1)
         if i >= args.warmup:
             vals.append(v)
+    if args.dump_outputs:
+        dump_gram(args.dump_outputs, info["gram"])
     vals.sort()
     value = vals[len(vals) // 2]                      # median over the timed steps
     nv = info["variants"]
@@ -424,6 +454,8 @@ def run_b200(args):
     barrier()
     clocks = sampler.stop()
     st1 = nat.stats()
+    if args.dump_outputs and rank == 0:
+        dump_gram(args.dump_outputs, nat.getGram())     # now: the kernel-only timing below leaves an unfinalized Gram
     ms = ev0.elapsed_time(ev1)
     if world > 1:
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
