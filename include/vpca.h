@@ -237,6 +237,48 @@ int vpca_get_centered(vpca_ctx* ctx, double* out);
 /* Tridiagonal form of the centered matrix after the last vpca_compute_pca (diag: n, offdiag: n-1). */
 int vpca_get_tridiagonal(vpca_ctx* ctx, double* diag, double* offdiag);
 
+/* ---- projection of held-out samples onto the fitted PCs -----------------------------------------------------------
+ * The reference fits every callset it reads (VariantsPca.scala:182-231).  A projecting context keeps N FITTED samples
+ * (cfg->n_samples; their Gram, centring and PCs are exactly what a plain N-sample context computes) and M PROJECTED ones
+ * that are only placed on those axes.  Rows of the context: fitted 0..N-1, projected N..N+M-1.
+ *   Cross counts  X_pf = #{variants where projected p and fitted f both carry variation}: the pair loop
+ *                 `for (c1 <- callset; c2 <- callset)` (:186-188) restricted to c1 projected, c2 fitted; exact int32 with the
+ *                 overflow bound of the Gram (:185).  Stored with the Gram in ONE (N+M) x N row-major buffer: rows 0..N-1
+ *                 the fitted Gram (the layout of a plain context), rows N..N+M-1 the cross block; the projected x projected
+ *                 counts are neither stored nor computed.  A caller-owned cfg->d_gram must hold (N+M) N int32.
+ *   Coordinates   the centring of :199-223 applied to a new row with the FITTED row sums and matrixMean, in the operation
+ *                 order of the fitted centring:  rs_p = sum_f X_pf (exact), rowMean_p = rs_p / N,
+ *                 c_pf = ((X_pf - rowMean_p) - rowSums_f / N) + matrixMean,   y_pc = (sum_f c_pf u_fc) / lambda_c
+ *                 (Gower's add-a-point formula).  The reference has no projection step: these numbers are not pinned by
+ *                 it.  Projected coordinates shrink towards 0 relative to fitted ones; no correction is applied.
+ * Input: every host-input and join route takes samples in SOURCE order and applies sample_rows on the device.  Pre-encoded
+ * input (vpca_accumulate_dense, vpca_accumulate_panels, the synthetic generator) has N+M rows already in row order.
+ * Existing entry points on a projecting context: get_gram / compute_pca / get_centered work on the fitted N x N block;
+ * get_partial_gram / load_partial_gram copy all (N+M) N counts; set_gram is VPCA_ERR_UNSUPPORTED, and so are
+ * vpca_gram_export_ipc / vpca_gram_set_peers / vpca_gram_set_peers_local (multi-GPU runs all-reduce the buffer of
+ * vpca_gram_device_ptr), gram_band_rows and VPCA_EXACT_COVER=1 (when M > 0).  The pool does not create projecting contexts. */
+typedef struct vpca_projection {
+    uint32_t struct_size;          /* sizeof(vpca_projection)                                                              */
+    int32_t n_projected;           /* M >= 0; M = 0 gives exactly the context vpca_create makes                           */
+    const int32_t* sample_rows;    /* N + M entries: input sample position s -> row of the context (fitted rows 0..N-1,
+                                      projected rows N..N+M-1); a permutation of 0..N+M-1, else VPCA_ERR_BAD_ARG.
+                                      NULL = identity (the last M inputs are projected).  Copied by the call.              */
+} vpca_projection;
+int vpca_create_projecting(const vpca_config* cfg, const vpca_projection* proj, vpca_ctx** out);
+/* The cross block X (M x N row-major int32) after vpca_finalize_gram: the rows of `matrix(c1, c2)` (:186-190) for c1
+ * projected.  M = 0: nothing is written. */
+int vpca_get_cross_gram(vpca_ctx* ctx, int32_t* out);
+/* Coordinates of the projected samples on the first k PCs of the last vpca_compute_pca (:224-227 extended to new rows):
+ * out[p + c * M] = y_pc, M x k column-major (the layout of vecs).  k <= the k of that call, else VPCA_ERR_BAD_ARG; before
+ * any vpca_compute_pca since the Gram last changed: VPCA_ERR_STATE.  Fixed reduction order: repeated calls are
+ * bit-identical. */
+int vpca_project_pca(vpca_ctx* ctx, int32_t k, double* out);
+/* Host-only: the tiles (records of vpca_debug_tiles) of a projecting context with n_fit fitted and n_total - n_fit
+ * projected samples -- A blocks over the n_fit columns of S, B rows over all n_total rows (row >= col); mxf4 != 0: the
+ * 240-wide strips of kind::mxf4, else the 256-wide ones of int8 / bf16.  Returns the tile count (may exceed max_tiles). */
+int vpca_debug_projection_tiles(int32_t n_fit, int32_t n_total, int32_t cta_group, int32_t mxf4, int32_t* out,
+                                int32_t max_tiles);
+
 /* ---- one process, all GPUs of the box (SURVEY 8b "process model") --------------------------------------------------
  * A vpca_pool is what `class VariantsPcaDriver` holds on a multi-GPU host: one vpca_ctx per GPU, wired with
  * vpca_gram_set_peers_local in VPCA_PEER_OWNER_ROWS mode (VPCA_PEER_REPLICATE when n_samples < 64 x n_gpus).  Spark

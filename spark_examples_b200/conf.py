@@ -112,4 +112,6 @@ class PcaConf(GenomicsConf):
             ("callsParquetPath", str, None, False),       # Parquet file of calls rows (parquet_calls.py): RDD[Seq[Int]] at rest
             ("bedPath", str, None, False),                # PLINK 1 fileset prefix (.bed/.bim/.fam) as the variants source
             ("bedCountedAllele", str, "A1", False),       # which .bim allele is "variation": A1 (PLINK's minor) or A2
+            ("projectedCallsets", str, None, False),      # file of callset names (one per line) placed on the PCs of the
+                                                          # others instead of being fitted (VariantsPcaDriver.projectPca)
         ]

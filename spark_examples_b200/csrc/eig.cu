@@ -63,9 +63,10 @@ __global__ void rowsum_kernel(const int32_t* __restrict__ S, int n, double* __re
     if (lane == 0) rowsum[row] = (double)acc;
 }
 
-// scal[0] = matrixMean (:211), nz = rowSums.filter(_ > 0).size (:207)
+// scal[0] = *mm = matrixMean (:211), nz = rowSums.filter(_ > 0).size (:207).  The solvers reuse scal as scratch; *mm is
+// what the projection of new rows reads.
 __global__ void matrix_mean_kernel(const double* __restrict__ rowsum, int n, double* __restrict__ scal,
-                                   int* __restrict__ nz) {
+                                   int* __restrict__ nz, double* __restrict__ mm) {
     __shared__ double red[33];
     __shared__ int cnt;
     if (threadIdx.x == 0) cnt = 0;
@@ -83,6 +84,7 @@ __global__ void matrix_mean_kernel(const double* __restrict__ rowsum, int n, dou
     if (threadIdx.x == 0) {
         const double rc = (double)n;
         scal[0] = __ddiv_rn(__ddiv_rn(tot, rc), rc);
+        *mm = scal[0];
         *nz = cnt;
     }
 }
@@ -1358,7 +1360,92 @@ __global__ void lz_lock_kernel(double* __restrict__ VT, int n, int cap, const do
     for (int c = 0; c < k; ++c) VT[(size_t)i * cap + c] = Z[(size_t)c * n + i];
 }
 
+// ------------------------------------------------------------------------------------------ projection
+// Coordinates of projected samples on the fitted PCs (Gower's add-a-point formula, the Nystrom extension of the centred
+// similarity): the cross row X_p (counts shared with every fitted sample, int32) is centred with the FITTED statistics in
+// the operation order of center_kernel (VariantsPca.scala:216-221 applied to a new row),
+//   c_pf = ((X_pf - rowMean_p) - rowSums_f / N) + matrixMean,   rowMean_p = (sum_f X_pf) / N,
+// and y_pc = (sum_f c_pf u_fc) / lambda_c.  Three launches, every reduction in a fixed order (no atomics): two calls give
+// bit-identical output.  The cross block is read twice -- the row sums must precede the centring -- but the second read
+// comes from L2 (the block of 2504 x 2504 counts is 25 MB).
+constexpr int kProjCols = 128;   // columns of S per block: 4 per lane, so a cohort of N samples makes ceil(N / 128) column
+                                 // chunks and even 50 projected rows fill ~140 blocks at N = 2504
+constexpr int kProjRows = 8;     // cross rows per block, one warp each
+
+__global__ void proj_rowmean_kernel(const int32_t* __restrict__ X, int n, int m, double* __restrict__ rowmean) {
+    const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (row >= m) return;
+    const int32_t* r = X + (size_t)row * n;
+    long long acc = 0;
+    for (int j = lane; j < n; j += 32) acc += r[j];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    // exact integer sum (the foldLeft(0D) of :206 on the new row), then rowMean as center_kernel forms it
+    if (lane == 0) rowmean[row] = __ddiv_rn((double)acc, (double)n);
+}
+
+// part[(q * m + p) * k + c] = sum over the columns f of chunk q of c_pf u_fc (ascending f per lane, then a fixed xor tree)
+__global__ void __launch_bounds__(32 * kProjRows) proj_dot_kernel(const int32_t* __restrict__ X, int n, int m,
+                                                                  const double* __restrict__ rowsum,
+                                                                  const double* __restrict__ mm,
+                                                                  const double* __restrict__ rowmean,
+                                                                  const double* __restrict__ U, int k,
+                                                                  double* __restrict__ part) {
+    const int q = blockIdx.x;
+    const int p = blockIdx.y * kProjRows + (int)(threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (p >= m) return;
+    const double rc = (double)n, rm = rowmean[p], mean = mm[0];
+    constexpr int kPer = kProjCols / 32;
+    double cv[kPer];
+#pragma unroll
+    for (int i = 0; i < kPer; ++i) {
+        const int f = q * kProjCols + i * 32 + lane;
+        cv[i] = 0.0;
+        if (f < n) {
+            const double data = lz_i2d(X[(size_t)p * n + f]);
+            cv[i] = __dadd_rn(__dsub_rn(__dsub_rn(data, rm), __ddiv_rn(rowsum[f], rc)), mean);
+        }
+    }
+    for (int c = 0; c < k; ++c) {
+        const double* u = U + (size_t)c * n;
+        double acc = 0.0;
+#pragma unroll
+        for (int i = 0; i < kPer; ++i) {
+            const int f = q * kProjCols + i * 32 + lane;
+            if (f < n) acc = __fma_rn(cv[i], u[f], acc);
+        }
+        acc = warp_sum(acc);
+        if (lane == 0) part[((size_t)q * m + p) * k + c] = acc;
+    }
+}
+
+// y[p + c * m] = (sum over chunks q in ascending order of part) / lambda_c
+__global__ void proj_finish_kernel(const double* __restrict__ part, int chunks, int m, int k,
+                                   const double* __restrict__ evals, double* __restrict__ y) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= m * k) return;
+    const int p = t / k, c = t - p * k;
+    double acc = 0.0;
+    for (int q = 0; q < chunks; ++q) acc = __dadd_rn(acc, part[((size_t)q * m + p) * k + c]);
+    y[p + (size_t)c * m] = __ddiv_rn(acc, evals[c]);
+}
+
 }  // namespace
+
+int proj_chunks(int n) { return (n + kProjCols - 1) / kProjCols; }
+
+cudaError_t eig_project(const EigWork& w, const int32_t* d_X, int m, int k, double* d_rowmean, double* d_part, double* d_y,
+                        cudaStream_t stream) {
+    if (m <= 0) return cudaSuccess;
+    const int n = w.n, chunks = proj_chunks(n);
+    proj_rowmean_kernel<<<(m + 7) / 8, 256, 0, stream>>>(d_X, n, m, d_rowmean);
+    proj_dot_kernel<<<dim3(chunks, (m + kProjRows - 1) / kProjRows), 32 * kProjRows, 0, stream>>>(
+        d_X, n, m, w.d_rowsum, w.d_mm, d_rowmean, w.d_evecs, k, d_part);
+    proj_finish_kernel<<<(m * k + 255) / 256, 256, 0, stream>>>(d_part, chunks, m, k, w.d_evals, d_y);
+    return cudaGetLastError();
+}
 
 cudaError_t eig_alloc(EigWork& w, int n, int kmax) {
     w.n = n;
@@ -1374,6 +1461,7 @@ cudaError_t eig_alloc(EigWork& w, int n, int kmax) {
     VPCA_TRY(cudaMalloc(&w.d_off, 2 * (size_t)n * sizeof(double)));   // e and e^2
     VPCA_TRY(cudaMalloc(&w.d_tau, (size_t)n * sizeof(double)));
     VPCA_TRY(cudaMalloc(&w.d_scal, 16 * sizeof(double)));
+    VPCA_TRY(cudaMalloc(&w.d_mm, sizeof(double)));
     VPCA_TRY(cudaMalloc(&w.d_evals, (size_t)kmax * sizeof(double)));
     VPCA_TRY(cudaMalloc(&w.d_evecs, (size_t)n * kmax * sizeof(double)));
     VPCA_TRY(cudaMalloc(&w.d_lu, 8 * (size_t)n * sizeof(double)));
@@ -1385,7 +1473,7 @@ cudaError_t eig_alloc(EigWork& w, int n, int kmax) {
 
 void eig_free(EigWork& w) {
     cudaFree(w.d_C); cudaFree(w.d_rowsum); cudaFree(w.d_v); cudaFree(w.d_w); cudaFree(w.d_p);
-    cudaFree(w.d_diag); cudaFree(w.d_off); cudaFree(w.d_tau); cudaFree(w.d_scal); cudaFree(w.d_evals);
+    cudaFree(w.d_diag); cudaFree(w.d_off); cudaFree(w.d_tau); cudaFree(w.d_scal); cudaFree(w.d_mm); cudaFree(w.d_evals);
     cudaFree(w.d_evecs); cudaFree(w.d_lu); cudaFree(w.d_nz); cudaFree(w.d_step);
     cudaFree(w.d_V); cudaFree(w.d_lzw); cudaFree(w.d_lzs); cudaFree(w.d_lzst); cudaFree(w.d_lzbar); cudaFree(w.d_lzprof); cudaFree(w.d_lzG);
     if (w.graph_exec != nullptr) cudaGraphExecDestroy(w.graph_exec);
@@ -1397,7 +1485,7 @@ cudaError_t center_gram(EigWork& w, const int32_t* d_S, cudaStream_t stream, boo
     const int n = w.n;
     w.d_S = d_S;   // the persistent Lanczos applies the centring to vectors and reads the int32 Gram itself
     rowsum_kernel<<<(n + 7) / 8, 256, 0, stream>>>(d_S, n, w.d_rowsum);
-    matrix_mean_kernel<<<1, 1024, 0, stream>>>(w.d_rowsum, n, w.d_scal, w.d_nz);
+    matrix_mean_kernel<<<1, 1024, 0, stream>>>(w.d_rowsum, n, w.d_scal, w.d_nz, w.d_mm);
     w.c_valid = false;
     if (materialise) return center_matrix(w, stream);
     return cudaGetLastError();

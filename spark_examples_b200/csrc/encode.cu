@@ -8,6 +8,9 @@
 // (row = sample, contiguous along variants) because that is the K-major operand layout the tcgen05 Gram kernel
 // streams through TMA.
 //
+// Projecting contexts hand a map `rows` (input sample position s -> row rows[s] of the tile; fitted samples first, then
+// projected ones): the cells of sample s land in row rows[s], so inputs stay in source order.  rows == nullptr: identity.
+//
 // HBM-bound scatter: one warp per variant row reads its indices coalesced and adds 1 to X[s][v] with a packed
 // 32-bit atomic (4 int8 cells or 2 bf16 cells per word), so duplicates and any index order are handled.
 #include <cuda_bf16.h>
@@ -30,7 +33,7 @@ __device__ __forceinline__ int64_t cell_index(int s, int64_t v, int64_t ld, int6
 template <typename IdxT>
 __global__ void encode_i8_kernel(const int64_t* __restrict__ off, int64_t base, const IdxT* __restrict__ idx,
                                  int64_t nv, int n, int max_mult, uint32_t* __restrict__ xw, int64_t ld,
-                                 int64_t panel, int* __restrict__ flags) {
+                                 int64_t panel, const int32_t* __restrict__ rows, int* __restrict__ flags) {
     const int lane = threadIdx.x & 31;
     const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     int bad = 0;
@@ -42,7 +45,7 @@ __global__ void encode_i8_kernel(const int64_t* __restrict__ off, int64_t base, 
                 bad |= 1;
                 continue;
             }
-            const int64_t byte = cell_index(s, v, ld, panel, n);
+            const int64_t byte = cell_index(rows != nullptr ? rows[s] : s, v, ld, panel, n);
             const uint32_t shift = (uint32_t)(byte & 3) * 8u;
             const uint32_t old = atomicAdd(xw + (byte >> 2), 1u << shift);
             if ((int)((old >> shift) & 0xFFu) >= max_mult) bad |= 2;
@@ -54,7 +57,7 @@ __global__ void encode_i8_kernel(const int64_t* __restrict__ off, int64_t base, 
 template <typename IdxT>
 __global__ void encode_bf16_kernel(const int64_t* __restrict__ off, int64_t base, const IdxT* __restrict__ idx,
                                    int64_t nv, int n, int max_mult, __nv_bfloat162* __restrict__ x2, int64_t ld,
-                                   int64_t panel, int* __restrict__ flags) {
+                                   int64_t panel, const int32_t* __restrict__ rows, int* __restrict__ flags) {
     const int lane = threadIdx.x & 31;
     const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     int bad = 0;
@@ -66,7 +69,7 @@ __global__ void encode_bf16_kernel(const int64_t* __restrict__ off, int64_t base
                 bad |= 1;
                 continue;
             }
-            const int64_t el = cell_index(s, v, ld, panel, n);
+            const int64_t el = cell_index(rows != nullptr ? rows[s] : s, v, ld, panel, n);
             const bool hi = (el & 1) != 0;
             const __nv_bfloat162 one = __floats2bfloat162_rn(hi ? 0.f : 1.f, hi ? 1.f : 0.f);
             const __nv_bfloat162 old = atomicAdd(x2 + (el >> 1), one);
@@ -82,7 +85,7 @@ __global__ void encode_bf16_kernel(const int64_t* __restrict__ off, int64_t base
 template <typename IdxT>
 __global__ void encode_e2m1_kernel(const int64_t* __restrict__ off, int64_t base, const IdxT* __restrict__ idx,
                                    int64_t nv, int n, int max_mult, uint32_t* __restrict__ xw, int64_t ld,
-                                   int64_t panel, int* __restrict__ flags) {
+                                   int64_t panel, const int32_t* __restrict__ rows, int* __restrict__ flags) {
     const int lane = threadIdx.x & 31;
     const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     int bad = 0;
@@ -94,7 +97,7 @@ __global__ void encode_e2m1_kernel(const int64_t* __restrict__ off, int64_t base
                 bad |= 1;
                 continue;
             }
-            const int64_t cell = cell_index(s, v, ld, panel, n);
+            const int64_t cell = cell_index(rows != nullptr ? rows[s] : s, v, ld, panel, n);
             const uint32_t shift = (uint32_t)(cell & 7) * 4u;
             const uint32_t old = atomicAdd(xw + (cell >> 3), 2u << shift);
             if ((int)((old >> shift) & 0xFu) >= 2 * max_mult) bad |= 2;
@@ -124,7 +127,8 @@ __device__ __forceinline__ uint32_t compress_even_bits(uint64_t x) {   // bit 2j
 
 template <int BITS>
 __global__ void bits_to_cells_kernel(const uint8_t* __restrict__ bits, int64_t stride, int64_t nv, int n,
-                                     uint8_t* __restrict__ x, int64_t ld, int64_t panel, int code) {
+                                     uint8_t* __restrict__ x, int64_t ld, int64_t panel, int code,
+                                     const int32_t* __restrict__ rows) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int words = (n + 31) / 32;                          // 32-sample words per variant
@@ -159,12 +163,13 @@ __global__ void bits_to_cells_kernel(const uint8_t* __restrict__ bits, int64_t s
     const int smp = k * 32 + lane;
     if (smp >= n) return;
     const int64_t v0 = vg * 32;
-    // cell index of (smp, v0): 32 consecutive cells never straddle a panel (panels are multiples of 128 cells)
+    const int row = rows != nullptr ? rows[smp] : smp;
+    // cell index of (row, v0): 32 consecutive cells never straddle a panel (panels are multiples of 128 cells)
     int64_t cell;
-    if (panel == 0) cell = (int64_t)smp * ld + v0;
+    if (panel == 0) cell = (int64_t)row * ld + v0;
     else {
         const int64_t pnl = v0 / panel;
-        cell = pnl * (int64_t)n * panel + (int64_t)smp * panel + (v0 - pnl * panel);
+        cell = pnl * (int64_t)n * panel + (int64_t)row * panel + (v0 - pnl * panel);
     }
     if constexpr (BITS == 8) {
         uint32_t o[8];
@@ -203,7 +208,7 @@ __global__ void bits_to_cells_kernel(const uint8_t* __restrict__ bits, int64_t s
 }  // namespace
 
 cudaError_t encode_bits(const uint8_t* d_bits, int64_t stride, int64_t nv, int n, int elem_bits, void* d_x, int64_t ld,
-                        int64_t panel, int code, cudaStream_t stream) {
+                        int64_t panel, int code, const int32_t* d_rows, cudaStream_t stream) {
     if (nv <= 0) return cudaSuccess;
     // every cell of the touched 32-variant groups is written, so only a partial last panel / k-block needs zeroing
     cudaError_t e = cudaSuccess;
@@ -223,31 +228,36 @@ cudaError_t encode_bits(const uint8_t* d_bits, int64_t stride, int64_t nv, int n
     const int threads = 256;
     const int64_t blocks = (warps * 32 + threads - 1) / threads;
     if (elem_bits == 8)
-        bits_to_cells_kernel<8><<<(unsigned)blocks, threads, 0, stream>>>(d_bits, stride, nv, n, static_cast<uint8_t*>(d_x), ld, panel, code);
+        bits_to_cells_kernel<8><<<(unsigned)blocks, threads, 0, stream>>>(d_bits, stride, nv, n, static_cast<uint8_t*>(d_x), ld, panel, code,
+                                                                          d_rows);
     else if (elem_bits == 4)
-        bits_to_cells_kernel<4><<<(unsigned)blocks, threads, 0, stream>>>(d_bits, stride, nv, n, static_cast<uint8_t*>(d_x), ld, panel, code);
+        bits_to_cells_kernel<4><<<(unsigned)blocks, threads, 0, stream>>>(d_bits, stride, nv, n, static_cast<uint8_t*>(d_x), ld, panel, code,
+                                                                          d_rows);
     else
-        bits_to_cells_kernel<16><<<(unsigned)blocks, threads, 0, stream>>>(d_bits, stride, nv, n, static_cast<uint8_t*>(d_x), ld, panel, code);
+        bits_to_cells_kernel<16><<<(unsigned)blocks, threads, 0, stream>>>(d_bits, stride, nv, n, static_cast<uint8_t*>(d_x), ld, panel, code,
+                                                                          d_rows);
     return cudaGetLastError();
 }
 
 template <typename IdxT>
 static cudaError_t encode_launch(const int64_t* d_off, int64_t base, const IdxT* d_idx, int64_t nv, int n, int elem_bits,
-                                 int max_mult, void* d_x, int64_t ld, int64_t panel, int* d_flags, cudaStream_t stream);
+                                 int max_mult, void* d_x, int64_t ld, int64_t panel, const int32_t* d_rows, int* d_flags,
+                                 cudaStream_t stream);
 
 cudaError_t encode_calls(const int64_t* d_off, int64_t base, const void* d_idx, int idx_bytes, int64_t nv, int n,
-                         int elem_bits, int max_mult, void* d_x, int64_t ld, int64_t panel, int* d_flags,
-                         cudaStream_t stream) {
+                         int elem_bits, int max_mult, void* d_x, int64_t ld, int64_t panel, const int32_t* d_rows,
+                         int* d_flags, cudaStream_t stream) {
     if (idx_bytes == 2)
         return encode_launch(d_off, base, static_cast<const uint16_t*>(d_idx), nv, n, elem_bits, max_mult, d_x, ld, panel,
-                             d_flags, stream);
-    return encode_launch(d_off, base, static_cast<const int32_t*>(d_idx), nv, n, elem_bits, max_mult, d_x, ld, panel, d_flags,
-                         stream);
+                             d_rows, d_flags, stream);
+    return encode_launch(d_off, base, static_cast<const int32_t*>(d_idx), nv, n, elem_bits, max_mult, d_x, ld, panel, d_rows,
+                         d_flags, stream);
 }
 
 template <typename IdxT>
 static cudaError_t encode_launch(const int64_t* d_off, int64_t base, const IdxT* d_idx, int64_t nv, int n, int elem_bits,
-                                 int max_mult, void* d_x, int64_t ld, int64_t panel, int* d_flags, cudaStream_t stream) {
+                                 int max_mult, void* d_x, int64_t ld, int64_t panel, const int32_t* d_rows, int* d_flags,
+                                 cudaStream_t stream) {
     cudaError_t e = cudaSuccess;
     if (panel > 0) {
         // whole panels are contiguous: zero every panel the rows touch
@@ -267,15 +277,15 @@ static cudaError_t encode_launch(const int64_t* d_off, int64_t base, const IdxT*
     if (elem_bits == 4) {
         const int cap = max_mult > 2 ? 2 : max_mult;
         encode_e2m1_kernel<IdxT><<<blocks, threads, 0, stream>>>(d_off, base, d_idx, nv, n, cap, reinterpret_cast<uint32_t*>(d_x),
-                                                           ld, panel, d_flags);
+                                                           ld, panel, d_rows, d_flags);
     } else if (elem_bits == 8) {
         const int cap = max_mult > 127 ? 127 : max_mult;
         encode_i8_kernel<IdxT><<<blocks, threads, 0, stream>>>(d_off, base, d_idx, nv, n, cap, reinterpret_cast<uint32_t*>(d_x), ld,
-                                                         panel, d_flags);
+                                                         panel, d_rows, d_flags);
     } else {
         const int cap = max_mult > 256 ? 256 : max_mult;   // bf16 holds integers exactly up to 256
         encode_bf16_kernel<IdxT><<<blocks, threads, 0, stream>>>(d_off, base, d_idx, nv, n, cap,
-                                                           reinterpret_cast<__nv_bfloat162*>(d_x), ld, panel, d_flags);
+                                                           reinterpret_cast<__nv_bfloat162*>(d_x), ld, panel, d_rows, d_flags);
     }
     return cudaGetLastError();
 }

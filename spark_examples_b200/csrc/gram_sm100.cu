@@ -25,6 +25,8 @@
 //     210 blocks instead of 220, 4.5 % less MMA work);
 //   * owner-computes bands: a context that stores only rows [own_lo, own_hi) of S and has no peers enumerates only the
 //     tiles of those rows (every variant is fed to every band's context; nothing is flushed anywhere else);
+//   * projecting contexts: X has N + M rows (fitted, then projected samples) and S has N columns at pitch N; the B strips
+//     run over all N + M rows, the A blocks over the N fitted ones, so rows N.. of S are the M x N cross block;
 //   * the variant axis is cut into k-blocks of 128 bytes (one swizzle atom) and into windows of `kb_window`
 //     k-blocks; in every window the (tile, k-block) units are split evenly over the workers (CTA pairs), and all
 //     workers walk the windows in the same order, so the slice of X a window needs (n x kb_window*128 B, sized to
@@ -102,7 +104,9 @@ struct GramArgs {
     int own_end[kMaxPeers];     // rank q owns Gram rows [own_end[q-1], own_end[q]); multiples of 32, >= 32 apart
     const TileDesc* tiles;
     int* err;          // mapped host memory: watchdog diagnostics
-    int n;
+    int n_cols;        // columns of S, also its row pitch: the fitted samples.  X may have more rows (projected samples,
+                       // rows n_cols .. row_limit - 1 of S); A blocks reaching past n_cols read them, and the guard
+                       // col < n_cols keeps those products out of S (at pitch n_cols they would land in the next row)
     int num_tiles;
     int num_full;      // leading tiles of full weight: what the large-N schedule deals out in whole-tile waves
     int total_weight;  // sum of n_eff / 16 over all tiles
@@ -603,22 +607,22 @@ __global__ void __launch_bounds__(kThreads, 1) gram_kernel(const __grid_constant
                 // rows (the even lane takes row 2 jj of both columns, the odd lane row 2 jj + 1), which halves the
                 // number of reds -- the L2 / NVLink atomic rate, not bytes, is what the flush runs against.  Needs an
                 // even row pitch (8-byte alignment of an even column); transposed chunks scatter and stay 32-bit.
-                if (!xpose && a.red64 != 0 && (a.n & 1) == 0) {
+                if (!xpose && a.red64 != 0 && (a.n_cols & 1) == 0) {
 #pragma unroll
                     for (int jj = 0; jj < 16; ++jj) {
                         const int row0 = rbase + 2 * jj, row1 = row0 + 1;
                         int v0, v1;
                         if constexpr (KIND == 0) { v0 = (int)r[2 * jj]; v1 = (int)r[2 * jj + 1]; }
                         else { v0 = __float2int_rn(__uint_as_float(r[2 * jj])); v1 = __float2int_rn(__uint_as_float(r[2 * jj + 1])); }
-                        if (!(row0 < row_end && col < a.n && row0 >= col)) v0 = 0;
-                        if (!(row1 < row_end && col < a.n && row1 >= col)) v1 = 0;
+                        if (!(row0 < row_end && col < a.n_cols && row0 >= col)) v0 = 0;
+                        if (!(row1 < row_end && col < a.n_cols && row1 >= col)) v1 = 0;
                         const int got = __shfl_xor_sync(0xffffffffu, (lane & 1) ? v0 : v1, 1);
                         const int srow = (lane & 1) ? row1 : row0;
                         const unsigned long long packed = (lane & 1)
                             ? ((unsigned long long)(unsigned)got | ((unsigned long long)(unsigned)v1 << 32))
                             : ((unsigned long long)(unsigned)v0 | ((unsigned long long)(unsigned)got << 32));
                         if (packed != 0ull) {
-                            const size_t o = (size_t)srow * (size_t)a.n + (size_t)(col & ~1);
+                            const size_t o = (size_t)srow * (size_t)a.n_cols + (size_t)(col & ~1);
                             if (a.num_peers == 0) {
                                 asm volatile("red.global.add.u64 [%0], %1;" ::"l"(a.S + o), "l"(packed) : "memory");
                             } else if (a.peer_mode == 1) {
@@ -636,14 +640,14 @@ __global__ void __launch_bounds__(kThreads, 1) gram_kernel(const __grid_constant
 #pragma unroll
                 for (int j = 0; j < 32; ++j) {
                     const int row = rbase + j;
-                    if (row < row_end && col < a.n && (xpose || row >= col)) {
+                    if (row < row_end && col < a.n_cols && (xpose || row >= col)) {
                         int v;
                         if constexpr (KIND == 0) v = (int)r[j];
                         else v = __float2int_rn(__uint_as_float(r[j]));
                         if (v != 0) {
                             // cell (srow, scol) of S: the lower-triangle position of this product
                             const int srow = xpose ? col : row, scol = xpose ? row : col;
-                            const size_t o = (size_t)srow * (size_t)a.n + (size_t)scol;
+                            const size_t o = (size_t)srow * (size_t)a.n_cols + (size_t)scol;
                             if (a.num_peers == 0) {
                                 asm volatile("red.global.add.s32 [%0], %1;" ::"l"(a.S + o), "r"(v) : "memory");
                             } else if (a.peer_mode == 1) {
@@ -932,9 +936,10 @@ cudaError_t launch(const CUtensorMap& tmap, const CUtensorMap& tmap_half, const 
 // list, window) starts from the split the last one ended with instead of relearning it over its first launches.
 namespace {
 struct SplitKey {
-    int dev, n, tiles, kbw, workers, elem;
+    int dev, n, rows, tiles, kbw, workers, elem;
     bool operator<(const SplitKey& o) const {
-        return std::tie(dev, n, tiles, kbw, workers, elem) < std::tie(o.dev, o.n, o.tiles, o.kbw, o.workers, o.elem);
+        return std::tie(dev, n, rows, tiles, kbw, workers, elem) <
+               std::tie(o.dev, o.n, o.rows, o.tiles, o.kbw, o.workers, o.elem);
     }
 };
 std::mutex g_split_mu;
@@ -950,7 +955,7 @@ static void remember_split(GramPlan& plan) {
         return;
     }
     std::lock_guard<std::mutex> lk(g_split_mu);
-    g_splits[SplitKey{plan.cum_dev, plan.cum_for_n, plan.cum_tiles, plan.cum_kbw, plan.cum_workers, plan.cum_elem}] = std::move(cum);
+    g_splits[SplitKey{plan.cum_dev, plan.cum_for_n, plan.cum_for_rows, plan.cum_tiles, plan.cum_kbw, plan.cum_workers, plan.cum_elem}] = std::move(cum);
 }
 
 void gram_plan_free(GramPlan& plan) {
@@ -1142,6 +1147,17 @@ int gram_debug_tiles(int n, int cta_group, int exact, int32_t* out, int max_tile
     return (int)tiles.size();
 }
 
+// Projecting context: A blocks over the n_fit columns of S, B strips over all n_total rows of X (row >= col).  For
+// n_total == n_fit this is exactly the tile list of a plain context.
+int gram_debug_projection_tiles(int n_fit, int n_total, int cta_group, bool mxf4, int32_t* out, int max_tiles) {
+    std::vector<TileDesc> tiles;
+    int num_full = 0;
+    make_tiles(n_fit, cta_group == 1 ? 1 : 2, false, mxf4 ? kUmmaNScaled : kUmmaN, 0, n_total, true, tiles, &num_full);
+    const int cnt = std::min<int>((int)tiles.size(), max_tiles);
+    if (out != nullptr && cnt > 0) memcpy(out, tiles.data(), (size_t)cnt * sizeof(TileDesc));
+    return (int)tiles.size();
+}
+
 int gram_debug_band_tiles(int n, int cta_group, int row_lo, int row_hi, int32_t* out, int max_tiles) {
     std::vector<TileDesc> tiles;
     int num_full = 0;
@@ -1186,8 +1202,8 @@ int gram_debug_repair(const int32_t* tiles8, int num_tiles, int workers, int kbw
     return cnt;
 }
 
-cudaError_t gram_accumulate(GramPlan& plan, const void* d_x, int elem_bits, int n, int64_t nv, int64_t ld, int64_t panel,
-                            int32_t* d_S, cudaStream_t stream, std::string* err) {
+cudaError_t gram_accumulate(GramPlan& plan, const void* d_x, int elem_bits, int n, int n_rows, int64_t nv, int64_t ld,
+                            int64_t panel, int32_t* d_S, cudaStream_t stream, std::string* err) {
     if (nv <= 0) return cudaSuccess;
     EncodeTiledFn encode = get_encode_fn();
     if (encode == nullptr) {
@@ -1240,8 +1256,12 @@ cudaError_t gram_accumulate(GramPlan& plan, const void* d_x, int elem_bits, int 
     // tiles of those rows are enumerated -- the caller feeds every variant of the cohort to every band's context and no
     // cell is produced twice anywhere (SURVEY 8e "shard output tiles across GPUs ... no reduction").
     const bool banded = plan.own_hi > plan.own_lo && plan.num_peers <= 1;
-    const int row_lo = banded ? plan.own_lo : 0, row_hi = banded ? plan.own_hi : n;
+    const int row_lo = banded ? plan.own_lo : 0, row_hi = banded ? plan.own_hi : n_rows;
     const bool exact = !mxf4 && plan.exact_cover && !banded;   // kind::mxf4 keeps 256 x 240 rectangles (block scales in TMEM)
+    if ((banded || exact || plan.num_peers > 1) && n_rows != n) {
+        if (err) *err = "projected rows need the rectangle tiling without peers or bands";
+        return cudaErrorNotSupported;
+    }
     if (plan.tiles_for_n != n || plan.tiles_for_cg != plan.cta_group || plan.tiles_for_bn != (exact ? -1 : tile_bn) ||
         plan.tiles_row_lo != row_lo || plan.tiles_row_hi != row_hi) {
         cudaError_t e = build_tiles(plan, n, exact, tile_bn, row_lo, row_hi, stream);
@@ -1277,9 +1297,10 @@ cudaError_t gram_accumulate(GramPlan& plan, const void* d_x, int elem_bits, int 
     // wide as the tile.  e2m1: globalDim[0] must be a multiple of 128 (the caller guarantees zero cells up to there).
     const int64_t npanels = panel > 0 ? (nv + panel - 1) / panel : 1;
     const int64_t dim0 = panel > 0 ? panel : (elem_bits == 4 ? (mxf4 ? ((nv + 1) / 2) * 2 : ((nv + 127) / 128) * 128) : nv);
-    const cuuint64_t gdim[3] = {(cuuint64_t)dim0, (cuuint64_t)n, (cuuint64_t)npanels};
+    // rows of X: all n_rows samples (fitted, then projected); S has n columns
+    const cuuint64_t gdim[3] = {(cuuint64_t)dim0, (cuuint64_t)n_rows, (cuuint64_t)npanels};
     const cuuint64_t gstride[2] = {(cuuint64_t)ld * (cuuint64_t)elem_bits / 8,
-                                   (cuuint64_t)n * (cuuint64_t)ld * (cuuint64_t)elem_bits / 8};
+                                   (cuuint64_t)n_rows * (cuuint64_t)ld * (cuuint64_t)elem_bits / 8};
     const cuuint32_t box[3] = {(cuuint32_t)elems_per_kb, (cuuint32_t)kBoxRows, 1};
     const cuuint32_t estr[3] = {1, 1, 1};
     const CUtensorMapDataType tmtype = elem_bits == 8 ? CU_TENSOR_MAP_DATA_TYPE_UINT8
@@ -1313,7 +1334,7 @@ cudaError_t gram_accumulate(GramPlan& plan, const void* d_x, int elem_bits, int 
     for (int d = 0; d < kMaxPeers; ++d) args.own_end[d] = plan.own_end[d];
     args.tiles = static_cast<const TileDesc*>(plan.d_tiles);
     cudaHostGetDevicePointer(reinterpret_cast<void**>(&args.err), plan.d_err, 0);
-    args.n = n;
+    args.n_cols = n;
     args.num_tiles = plan.num_tiles;
     args.num_full = plan.num_full;
     args.total_weight = plan.total_weight;
@@ -1331,7 +1352,7 @@ cudaError_t gram_accumulate(GramPlan& plan, const void* d_x, int elem_bits, int 
         if (kbw <= 0) {
             // window of X sized to ~32 MiB so that every tile re-reads it from L2 (126 MB) rather than HBM
             const long long target = 32ll << 20;
-            kbw = (int)std::max<long long>(8, std::min<long long>(4096, target / ((long long)n * kKBytes)));
+            kbw = (int)std::max<long long>(8, std::min<long long>(4096, target / ((long long)n_rows * kKBytes)));
         }
         kbw = std::min(kbw, args.kb_total);
         // cheap upper bound first (a worker with less than a tile's worth of work can touch few tiles), then the exact test
@@ -1343,11 +1364,12 @@ cudaError_t gram_accumulate(GramPlan& plan, const void* d_x, int elem_bits, int 
         // the device-side split (speed-weighted by rebalance_kernel from launch to launch) starts from the repaired
         // equal split; it is only meaningful for one (workers, tile list, window length)
         if (args.resident && (plan.d_cum == nullptr || plan.cum_workers != workers || plan.cum_tiles != plan.num_tiles ||
-                              plan.cum_kbw != kbw || plan.cum_for_n != n || plan.cum_elem != elem_bits)) {
+                              plan.cum_kbw != kbw || plan.cum_for_n != n || plan.cum_for_rows != n_rows ||
+                              plan.cum_elem != elem_bits)) {
             remember_split(plan);
             if (plan.adaptive && !banded) {   // a split learned earlier on this device for the same schedule, if it still fits TMEM
                 std::lock_guard<std::mutex> lk(g_split_mu);
-                auto it = g_splits.find(SplitKey{dev, n, plan.num_tiles, kbw, workers, elem_bits});
+                auto it = g_splits.find(SplitKey{dev, n, n_rows, plan.num_tiles, kbw, workers, elem_bits});
                 if (it != g_splits.end()) {
                     std::vector<double> learned = it->second;
                     const TileDesc* tiles = reinterpret_cast<const TileDesc*>(plan.h_tiles.data());
@@ -1369,6 +1391,7 @@ cudaError_t gram_accumulate(GramPlan& plan, const void* d_x, int elem_bits, int 
             plan.cum_tiles = plan.num_tiles;
             plan.cum_kbw = kbw;
             plan.cum_for_n = n;
+            plan.cum_for_rows = n_rows;
             plan.cum_dev = dev;
             plan.cum_elem = elem_bits;
         }

@@ -43,6 +43,15 @@ struct vpca_ctx {
     int32_t* d_S = nullptr;
     bool own_S = false;
     int band_row0 = 0, band_rows = 0;   // rows of the Gram this context stores (band_rows == n: all of them)
+    // projecting context (vpca_create_projecting): n_proj samples beyond the n fitted ones.  The Gram buffer is
+    // (n + n_proj) x n, pitch n: rows [0, n) the fitted Gram, rows [n, n + n_proj) the cross block.  Input sample s is
+    // row d_rows[s] of the genotype tiles (d_rows == nullptr: identity).
+    int n_proj = 0;
+    int32_t* d_rows = nullptr;
+    int proj_k = 0;                // k of the last vpca_compute_pca (0: none since the Gram last changed)
+    double* d_proj = nullptr;      // projection scratch + result (eig_project)
+    int rows() const { return n + n_proj; }                                        // rows of X
+    size_t gram_cells() const { return (size_t)(band_rows + n_proj) * (size_t)n; }   // int32 cells of d_S
     bool finalized = false;
     bool pca_done = false;
     GramPlan plan;        // schedule state of the launches on `stream` (device-resident input)
@@ -181,7 +190,7 @@ void sync_peers_to_lanes(vpca_ctx* ctx) {
 
 void staging_geometry(vpca_ctx* ctx) {
     if (ctx->chunk_variants != 0) return;
-    const int n = ctx->n, bits = ctx->elem_bits;
+    const int n = ctx->rows(), bits = ctx->elem_bits;
     int64_t cv = ctx->cfg.chunk_variants;
     if (cv <= 0) {
         cv = (256ll << 20) * 8 / ((int64_t)n * bits);
@@ -203,7 +212,7 @@ void staging_geometry(vpca_ctx* ctx) {
 // later call retries from scratch instead of running on half a lane.
 int ensure_lane(vpca_ctx* ctx, vpca_ctx::Lane& L) {
     if (L.ready) return VPCA_OK;
-    const int n = ctx->n, bits = ctx->elem_bits;
+    const int n = ctx->rows(), bits = ctx->elem_bits;
     const int64_t cv = ctx->chunk_variants, cz = ctx->chunk_nnz;
     cudaError_t e = cudaStreamCreateWithFlags(&L.stream, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&L.copy_stream, cudaStreamNonBlocking);
@@ -283,10 +292,10 @@ int launch_gram(vpca_ctx* ctx, GramPlan& plan, cudaStream_t stream, cudaEvent_t 
         std::string msg;
         cudaEventRecord(t0, stream);
         // sub-launches start on a panel boundary (panel layout) or at column v0 (row-major)
-        const size_t byte_off = panel > 0 ? (size_t)(v0 / panel) * (size_t)ctx->n * (size_t)panel * ctx->elem_bits / 8
+        const size_t byte_off = panel > 0 ? (size_t)(v0 / panel) * (size_t)ctx->rows() * (size_t)panel * ctx->elem_bits / 8
                                           : (size_t)v0 * ctx->elem_bits / 8;
-        cudaError_t e = gram_accumulate(plan, static_cast<const char*>(d_x) + byte_off, ctx->elem_bits, ctx->n, cnt, ld,
-                                        panel, d_target, stream, &msg);
+        cudaError_t e = gram_accumulate(plan, static_cast<const char*>(d_x) + byte_off, ctx->elem_bits, ctx->n, ctx->rows(),
+                                        cnt, ld, panel, d_target, stream, &msg);
         cudaEventRecord(t1, stream);
         if (e != cudaSuccess)
             return fail(ctx, VPCA_ERR_CUDA, "Gram launch failed: %s %s", cudaGetErrorString(e), msg.c_str());
@@ -305,7 +314,7 @@ vpca_ctx::Slot* find_slot(vpca_ctx* ctx, int64_t pid, bool create, int* rc) {
     for (auto& s : ctx->slots)
         if (!s.used) {
             if (s.d_S == nullptr) {
-                cudaError_t e = cudaMalloc(&s.d_S, (size_t)ctx->n * ctx->n * sizeof(int32_t));
+                cudaError_t e = cudaMalloc(&s.d_S, (size_t)ctx->rows() * ctx->n * sizeof(int32_t));
                 if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.ev_free, cudaEventDisableTiming);
                 if (e != cudaSuccess) {
                     cudaFree(s.d_S);
@@ -386,7 +395,7 @@ struct CallScope {
 int prepare_slot(vpca_ctx* ctx, vpca_ctx::Lane& L, CallScope& sc) {
     if (sc.slot == nullptr || !sc.fresh) return VPCA_OK;
     CUDA_OK(ctx, cudaStreamWaitEvent(L.stream, sc.slot->ev_free, 0));
-    CUDA_OK(ctx, cudaMemsetAsync(sc.slot->d_S, 0, (size_t)ctx->n * ctx->n * sizeof(int32_t), L.stream));
+    CUDA_OK(ctx, cudaMemsetAsync(sc.slot->d_S, 0, (size_t)ctx->rows() * ctx->n * sizeof(int32_t), L.stream));
     return VPCA_OK;
 }
 
@@ -441,8 +450,8 @@ int process_calls(vpca_ctx* ctx, vpca_ctx::Lane& L, const int64_t* offsets, cons
         ctx->c_h2d += (nvc + 1) * 8 + nnz * idx_bytes;
         CUDA_OK(ctx, cudaStreamWaitEvent(L.stream, L.ev_copy[b], 0));
         const int64_t P = ctx->panel;
-        CUDA_OK(ctx, encode_calls(L.d_off[b], offsets[v], L.d_idx[b], idx_bytes, nvc, ctx->n, bits, ctx->max_mult, L.d_x[b], P, P,
-                                  L.d_flags, L.stream));
+        CUDA_OK(ctx, encode_calls(L.d_off[b], offsets[v], L.d_idx[b], idx_bytes, nvc, ctx->rows(), bits, ctx->max_mult, L.d_x[b],
+                                  P, P, ctx->d_rows, L.d_flags, L.stream));
         ctx->c_launches += 2;
         if (out_tile != nullptr) {
             // panel layout -> the caller's row-major tile, one 2-D copy per panel (chunk boundaries are multiples of
@@ -451,11 +460,11 @@ int process_calls(vpca_ctx* ctx, vpca_ctx::Lane& L, const int64_t* offsets, cons
                 const int64_t wv = std::min(P, nvc - pv);
                 CUDA_OK(ctx, cudaMemcpy2DAsync(static_cast<char*>(out_tile) + (size_t)(v + pv) * bits / 8,
                                                (size_t)out_ld * bits / 8,
-                                               static_cast<const char*>(L.d_x[b]) + (size_t)(pv / P) * ctx->n * P * bits / 8,
-                                               (size_t)P * bits / 8, (size_t)(wv * bits + 7) / 8, (size_t)ctx->n,
+                                               static_cast<const char*>(L.d_x[b]) + (size_t)(pv / P) * ctx->rows() * P * bits / 8,
+                                               (size_t)P * bits / 8, (size_t)(wv * bits + 7) / 8, (size_t)ctx->rows(),
                                                cudaMemcpyDeviceToHost, L.stream));
             }
-            ctx->c_d2h += (nvc * bits + 7) / 8 * (int64_t)ctx->n;
+            ctx->c_d2h += (nvc * bits + 7) / 8 * (int64_t)ctx->rows();
         } else {
             int rc = launch_gram(ctx, L.plan, L.stream, L.ev_t0, L.ev_t1, L.d_x[b], nvc, P, P, d_target);
             if (rc != VPCA_OK) return rc;
@@ -471,7 +480,7 @@ int process_calls(vpca_ctx* ctx, vpca_ctx::Lane& L, const int64_t* offsets, cons
     if (launched) lane_gram_time(ctx, L);
     if (*L.h_flags & 1)
         return fail(ctx, VPCA_ERR_INDEX_OUT_OF_RANGE, "sample index outside [0, %d) (the reference throws at "
-                    "VariantsPca.scala:59/:188)", ctx->n);
+                    "VariantsPca.scala:59/:188)", ctx->rows());
     if (*L.h_flags & 2)
         return fail(ctx, VPCA_ERR_OVERFLOW, "a sample is listed more than max_multiplicity=%d times in one row",
                     ctx->max_mult);
@@ -506,7 +515,7 @@ const char* vpca_last_error(const vpca_ctx* ctx) {
     return tls_error_copy.c_str();
 }
 
-int vpca_create(const vpca_config* cfg, vpca_ctx** out) {
+static int create_impl(const vpca_config* cfg, int n_proj, const int32_t* sample_rows, vpca_ctx** out) {
     if (out == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "out is NULL");
     *out = nullptr;
     if (cfg == nullptr || cfg->struct_size != sizeof(vpca_config))
@@ -532,6 +541,7 @@ int vpca_create(const vpca_config* cfg, vpca_ctx** out) {
     if (ctx == nullptr) return fail(nullptr, VPCA_ERR_NOMEM, "out of host memory");
     ctx->cfg = *cfg;
     ctx->n = cfg->n_samples;
+    ctx->n_proj = n_proj;
     ctx->elem_bits = cfg->dtype == VPCA_DTYPE_I8 ? 8 : (cfg->dtype == VPCA_DTYPE_BF16 ? 16 : 4);
     ctx->max_mult = cfg->max_multiplicity > 0 ? cfg->max_multiplicity : 2;
     ctx->num_pc = cfg->num_pc > 0 ? cfg->num_pc : 2;
@@ -564,7 +574,7 @@ int vpca_create(const vpca_config* cfg, vpca_ctx** out) {
         e = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking);
         ctx->own_stream = true;
     }
-    const size_t gram_cells = (size_t)ctx->band_rows * ctx->n;
+    const size_t gram_cells = ctx->gram_cells();
     if (e == cudaSuccess) {
         if (cfg->d_gram != nullptr) {
             ctx->d_S = static_cast<int32_t*>(cfg->d_gram);
@@ -575,6 +585,11 @@ int vpca_create(const vpca_config* cfg, vpca_ctx** out) {
         }
     }
     if (e == cudaSuccess) e = cudaMemsetAsync(ctx->d_S, 0, gram_cells * sizeof(int32_t), ctx->stream);
+    if (e == cudaSuccess && sample_rows != nullptr) {
+        e = cudaMalloc(&ctx->d_rows, (size_t)ctx->rows() * sizeof(int32_t));
+        if (e == cudaSuccess)
+            e = cudaMemcpy(ctx->d_rows, sample_rows, (size_t)ctx->rows() * sizeof(int32_t), cudaMemcpyHostToDevice);
+    }
     if (e == cudaSuccess) e = cudaEventCreate(&ctx->ev_t0);
     if (e == cudaSuccess) e = cudaEventCreate(&ctx->ev_t1);
     if (e == cudaSuccess) e = cudaEventCreate(&ctx->ev_e0);
@@ -592,6 +607,42 @@ int vpca_create(const vpca_config* cfg, vpca_ctx** out) {
     return VPCA_OK;
 }
 
+int vpca_create(const vpca_config* cfg, vpca_ctx** out) { return create_impl(cfg, 0, nullptr, out); }
+
+int vpca_create_projecting(const vpca_config* cfg, const vpca_projection* proj, vpca_ctx** out) {
+    if (out != nullptr) *out = nullptr;
+    if (proj == nullptr || proj->struct_size != sizeof(vpca_projection))
+        return fail(nullptr, VPCA_ERR_BAD_ARG, "proj is NULL or struct_size != sizeof(vpca_projection) (%zu)",
+                    sizeof(vpca_projection));
+    if (cfg == nullptr || cfg->struct_size != sizeof(vpca_config))
+        return fail(nullptr, VPCA_ERR_BAD_ARG, "cfg is NULL or struct_size != sizeof(vpca_config) (%zu)", sizeof(vpca_config));
+    const int m = proj->n_projected;
+    if (m < 0 || (int64_t)cfg->n_samples + m > 0x7fffffff)
+        return fail(nullptr, VPCA_ERR_BAD_ARG, "n_projected must be >= 0 and n_samples + n_projected < 2^31");
+    const int total = cfg->n_samples + m;
+    bool identity = true;
+    if (proj->sample_rows != nullptr && cfg->n_samples >= 0) {
+        std::vector<char> seen((size_t)total, 0);
+        for (int s = 0; s < total; ++s) {
+            const int32_t r = proj->sample_rows[s];
+            if (r < 0 || r >= total || seen[(size_t)r])
+                return fail(nullptr, VPCA_ERR_BAD_ARG, "sample_rows is not a permutation of [0, %d): entry %d is %d", total, s, r);
+            seen[(size_t)r] = 1;
+            identity = identity && r == s;
+        }
+    }
+    if (m > 0) {
+        // Out of scope for projection: fused peer reductions (refused by vpca_gram_set_peers*), row bands and the exact
+        // block cover (the cross block needs the rectangle tiling)
+        if (cfg->gram_band_rows > 0)
+            return fail(nullptr, VPCA_ERR_UNSUPPORTED, "a projecting context stores the whole fitted Gram (no gram_band_rows)");
+        const char* ex = getenv("VPCA_EXACT_COVER");
+        if (ex != nullptr && atoi(ex) != 0)
+            return fail(nullptr, VPCA_ERR_UNSUPPORTED, "VPCA_EXACT_COVER=1 has no tiling of the cross block");
+    }
+    return create_impl(cfg, m, identity ? nullptr : proj->sample_rows, out);
+}
+
 int vpca_destroy(vpca_ctx* ctx) {
     if (ctx == nullptr) return VPCA_OK;
     cudaSetDevice(ctx->cfg.device);
@@ -605,6 +656,8 @@ int vpca_destroy(vpca_ctx* ctx) {
         for (int d = 0; d < ctx->plan.num_peers; ++d)
             if (d != ctx->plan.peer_rank && ctx->plan.peer_S[d] != nullptr) cudaIpcCloseMemHandle(ctx->plan.peer_base[d]);
     if (ctx->own_S) cudaFree(ctx->d_S);
+    cudaFree(ctx->d_rows);
+    cudaFree(ctx->d_proj);
     if (ctx->eig_ready) eig_free(ctx->eig);
     join_free(ctx->join);
     gram_plan_free(ctx->plan);
@@ -629,10 +682,11 @@ int vpca_reset(vpca_ctx* ctx) {
     for (auto& L : ctx->lanes)
         if (L.busy) return fail(ctx, VPCA_ERR_STATE, "vpca_reset while an accumulate call is in flight");
     CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
-    CUDA_OK(ctx, cudaMemsetAsync(ctx->d_S, 0, (size_t)ctx->band_rows * ctx->n * sizeof(int32_t), ctx->stream));
+    CUDA_OK(ctx, cudaMemsetAsync(ctx->d_S, 0, ctx->gram_cells() * sizeof(int32_t), ctx->stream));
     for (auto& s : ctx->slots) s.used = false;
     ctx->finalized = false;
     ctx->pca_done = false;
+    ctx->proj_k = 0;
     ctx->total_variants = 0;
     ctx->inflight_variants = 0;
     ctx->st.variants_accumulated = 0;
@@ -682,7 +736,8 @@ int vpca_accumulate_calls(vpca_ctx* ctx, int64_t partition_id, const int64_t* of
 
 int vpca_accumulate_calls_u16(vpca_ctx* ctx, int64_t partition_id, const int64_t* offsets, const uint16_t* sample_idx,
                               int64_t nv) {
-    if (ctx != nullptr && ctx->n > 65536) return fail(ctx, VPCA_ERR_BAD_ARG, "16-bit sample indices need n_samples <= 65536");
+    if (ctx != nullptr && ctx->rows() > 65536)
+        return fail(ctx, VPCA_ERR_BAD_ARG, "16-bit sample indices need n_samples (+ n_projected) <= 65536");
     return accumulate_calls_impl(ctx, partition_id, offsets, sample_idx, 2, nv);
 }
 
@@ -690,7 +745,7 @@ int vpca_accumulate_calls_u16(vpca_ctx* ctx, int64_t partition_id, const int64_t
 static int accumulate_packed(vpca_ctx* ctx, int64_t partition_id, const uint8_t* bits, int64_t nv, int64_t stride_bytes,
                              int code) {
     if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
-    const int64_t min_stride = code == 0 ? (ctx->n + 7) / 8 : (ctx->n + 3) / 4;
+    const int64_t min_stride = code == 0 ? (ctx->rows() + 7) / 8 : (ctx->rows() + 3) / 4;
     if (nv < 0 || (nv > 0 && bits == nullptr) || stride_bytes < min_stride)
         return fail(ctx, VPCA_ERR_BAD_ARG, "packed rows: stride_bytes must be >= ceil(n_samples / %d)", code == 0 ? 8 : 4);
     CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
@@ -722,8 +777,8 @@ static int accumulate_packed(vpca_ctx* ctx, int64_t partition_id, const uint8_t*
             CUDA_OK(ctx, cudaEventRecord(L.ev_copy[b], L.copy_stream));
             ctx->c_h2d += nvc * stride_bytes;
             CUDA_OK(ctx, cudaStreamWaitEvent(L.stream, L.ev_copy[b], 0));
-            CUDA_OK(ctx, encode_bits(reinterpret_cast<const uint8_t*>(L.d_idx[b]), stride_bytes, nvc, ctx->n, ctx->elem_bits,
-                                     L.d_x[b], P, P, code, L.stream));
+            CUDA_OK(ctx, encode_bits(reinterpret_cast<const uint8_t*>(L.d_idx[b]), stride_bytes, nvc, ctx->rows(), ctx->elem_bits,
+                                     L.d_x[b], P, P, code, ctx->d_rows, L.stream));
             ctx->c_launches += 1;
             r = launch_gram(ctx, L.plan, L.stream, L.ev_t0, L.ev_t1, L.d_x[b], nvc, P, P, sc.target);
             if (r != VPCA_OK) return r;
@@ -893,8 +948,8 @@ int vpca_accumulate_joined(vpca_ctx* ctx, int64_t partition_id) {
             const int64_t nvc = std::min(ctx->chunk_variants, nv - v);
             const int b = chunk & 1;
             // the joined CSR is device-resident: rows [v, v + nvc) are encoded straight from it (absolute offsets, base 0)
-            CUDA_OK(ctx, encode_calls(w.d_out_off + v, 0, w.d_out_idx, 4, nvc, ctx->n, ctx->elem_bits, ctx->max_mult, L.d_x[b],
-                                      P, P, L.d_flags, L.stream));
+            CUDA_OK(ctx, encode_calls(w.d_out_off + v, 0, w.d_out_idx, 4, nvc, ctx->rows(), ctx->elem_bits, ctx->max_mult,
+                                      L.d_x[b], P, P, ctx->d_rows, L.d_flags, L.stream));
             ctx->c_launches += 2;
             r = launch_gram(ctx, L.plan, L.stream, L.ev_t0, L.ev_t1, L.d_x[b], nvc, P, P, sc.target);
             if (r != VPCA_OK) return r;
@@ -904,7 +959,7 @@ int vpca_accumulate_joined(vpca_ctx* ctx, int64_t partition_id) {
         lane_gram_time(ctx, L);
         if (*L.h_flags & 1)
             return fail(ctx, VPCA_ERR_INDEX_OUT_OF_RANGE, "sample index outside [0, %d) (the reference throws at "
-                        "VariantsPca.scala:59/:188)", ctx->n);
+                        "VariantsPca.scala:59/:188)", ctx->rows());
         if (*L.h_flags & 2)
             return fail(ctx, VPCA_ERR_OVERFLOW, "a sample is listed more than max_multiplicity=%d times in one joined row "
                         "(a sample present in both datasets counts twice, VariantsPca.scala:127/:187)", ctx->max_mult);
@@ -935,7 +990,7 @@ int vpca_commit(vpca_ctx* ctx, int64_t partition_id) {
         else if (ctx->plan.num_peers > 1)
             CUDA_OK(ctx, gram_add_peers(ctx->plan, s->d_S, (int64_t)ctx->n * ctx->n, ctx->stream));
         else
-            CUDA_OK(ctx, gram_add(ctx->d_S, s->d_S, (int64_t)ctx->n * ctx->n, ctx->stream));
+            CUDA_OK(ctx, gram_add(ctx->d_S, s->d_S, (int64_t)ctx->rows() * ctx->n, ctx->stream));
         CUDA_OK(ctx, cudaEventRecord(s->ev_free, ctx->stream));
         ctx->c_launches += 1;
     }
@@ -998,17 +1053,17 @@ int vpca_accumulate_dense(vpca_ctx* ctx, const void* x, int64_t nv, int64_t ld, 
             // the caller's row-major tile -> panel layout, one 2-D copy per panel; a partial last panel is zeroed first
             const int64_t P = ctx->panel;
             if ((nvc % P) != 0)
-                CUDA_OK(ctx, cudaMemsetAsync(static_cast<char*>(L.d_x[b]) + (size_t)(nvc / P) * ctx->n * P * bits / 8, 0,
-                                             (size_t)ctx->n * P * bits / 8, L.copy_stream));
+                CUDA_OK(ctx, cudaMemsetAsync(static_cast<char*>(L.d_x[b]) + (size_t)(nvc / P) * ctx->rows() * P * bits / 8, 0,
+                                             (size_t)ctx->rows() * P * bits / 8, L.copy_stream));
             for (int64_t pv = 0; pv < nvc; pv += P) {
                 const int64_t wv = std::min(P, nvc - pv);
-                CUDA_OK(ctx, cudaMemcpy2DAsync(static_cast<char*>(L.d_x[b]) + (size_t)(pv / P) * ctx->n * P * bits / 8,
+                CUDA_OK(ctx, cudaMemcpy2DAsync(static_cast<char*>(L.d_x[b]) + (size_t)(pv / P) * ctx->rows() * P * bits / 8,
                                                (size_t)P * bits / 8, static_cast<const char*>(x) + (size_t)(v + pv) * bits / 8,
-                                               (size_t)ld * bits / 8, (size_t)(wv * bits + 7) / 8, (size_t)ctx->n,
+                                               (size_t)ld * bits / 8, (size_t)(wv * bits + 7) / 8, (size_t)ctx->rows(),
                                                cudaMemcpyHostToDevice, L.copy_stream));
             }
             CUDA_OK(ctx, cudaEventRecord(L.ev_copy[b], L.copy_stream));
-            ctx->c_h2d += (nvc * bits + 7) / 8 * (int64_t)ctx->n;
+            ctx->c_h2d += (nvc * bits + 7) / 8 * (int64_t)ctx->rows();
             CUDA_OK(ctx, cudaStreamWaitEvent(L.stream, L.ev_copy[b], 0));
             int r = launch_gram(ctx, L.plan, L.stream, L.ev_t0, L.ev_t1, L.d_x[b], nvc, P, P, ctx->d_S);
             if (r != VPCA_OK) return r;
@@ -1059,7 +1114,7 @@ int vpca_synth_panels_device(vpca_ctx* ctx, uint64_t seed, int64_t v0, int64_t n
         return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_synth_panels_device: bad argument");
     if (mode == 1 && ctx->max_mult < 2) return fail(ctx, VPCA_ERR_BAD_ARG, "dosage mode needs max_multiplicity >= 2");
     CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
-    cudaError_t e = synth_dense(seed, ctx->n, v0, nv, mode, ctx->elem_bits, d_x, panel_variants, panel_variants, ctx->stream);
+    cudaError_t e = synth_dense(seed, ctx->rows(), v0, nv, mode, ctx->elem_bits, d_x, panel_variants, panel_variants, ctx->stream);
     if (e != cudaSuccess) return fail(ctx, VPCA_ERR_CUDA, "synthetic generator: %s", cudaGetErrorString(e));
     ctx->c_launches += 2 * ((nv + (1 << 22) - 1) >> 22);
     return VPCA_OK;
@@ -1087,6 +1142,7 @@ int vpca_finalize_gram(vpca_ctx* ctx) {
     }
     ctx->finalized = true;
     ctx->pca_done = false;
+    ctx->proj_k = 0;
     return VPCA_OK;
 }
 
@@ -1127,7 +1183,7 @@ int vpca_get_partial_gram(vpca_ctx* ctx, int32_t* out, int64_t* variants_in_gram
     if (ctx->finalized) return fail(ctx, VPCA_ERR_STATE, "Gram already finalized: use vpca_get_gram");
     if (ctx->band_rows != ctx->n) return fail(ctx, VPCA_ERR_STATE, "this context stores a row band: use vpca_get_gram_band");
     if (variants_in_gram) *variants_in_gram = ctx->total_variants;
-    return copy_gram_out(ctx, out, (size_t)ctx->n * ctx->n);
+    return copy_gram_out(ctx, out, ctx->gram_cells());
 }
 
 int vpca_load_partial_gram(vpca_ctx* ctx, const int32_t* gram, int64_t variants_in_gram) {
@@ -1138,7 +1194,7 @@ int vpca_load_partial_gram(vpca_ctx* ctx, const int32_t* gram, int64_t variants_
     for (auto& s : ctx->slots)
         if (s.used) return fail(ctx, VPCA_ERR_STATE, "partition %lld is in flight", (long long)s.pid);
     CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
-    const size_t bytes = (size_t)ctx->n * ctx->n * sizeof(int32_t);
+    const size_t bytes = ctx->gram_cells() * sizeof(int32_t);
     CUDA_OK(ctx, cudaMemcpyAsync(ctx->d_S, gram, bytes, cudaMemcpyHostToDevice, ctx->stream));
     CUDA_OK(ctx, cudaStreamSynchronize(ctx->stream));
     ctx->c_h2d += (int64_t)bytes;
@@ -1152,6 +1208,9 @@ int vpca_set_gram(vpca_ctx* ctx, const int32_t* gram) {
     if (ctx == nullptr || gram == nullptr) return fail(ctx, VPCA_ERR_BAD_ARG, "NULL argument");
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (ctx->band_rows != ctx->n) return fail(ctx, VPCA_ERR_STATE, "this context stores a row band");
+    if (ctx->n_proj > 0)
+        return fail(ctx, VPCA_ERR_UNSUPPORTED, "a projecting context computes its cross block from genotypes: vpca_set_gram "
+                    "would leave it stale");
     CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
     const size_t bytes = (size_t)ctx->n * ctx->n * sizeof(int32_t);
     CUDA_OK(ctx, cudaMemcpyAsync(ctx->d_S, gram, bytes, cudaMemcpyHostToDevice, ctx->stream));
@@ -1218,7 +1277,59 @@ int vpca_compute_pca(vpca_ctx* ctx, int32_t k, double* vecs, double* evals, int3
     if (non_zero_rows) *non_zero_rows = nz;
     ctx->c_d2h += (int64_t)nb + (evals ? k * 8 : 0) + 4;
     ctx->pca_done = true;
+    ctx->proj_k = k;
     return VPCA_OK;
+}
+
+int vpca_get_cross_gram(vpca_ctx* ctx, int32_t* out) {
+    if (ctx == nullptr || out == nullptr) return fail(ctx, VPCA_ERR_BAD_ARG, "NULL argument");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (!ctx->finalized) return fail(ctx, VPCA_ERR_STATE, "call vpca_finalize_gram first");
+    if (ctx->n_proj == 0) return VPCA_OK;
+    CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
+    const size_t cells = (size_t)ctx->n_proj * ctx->n;
+    CUDA_OK(ctx, cudaMemcpyAsync(out, ctx->d_S + (size_t)ctx->n * ctx->n, cells * sizeof(int32_t), cudaMemcpyDeviceToHost,
+                                 ctx->stream));
+    CUDA_OK(ctx, cudaStreamSynchronize(ctx->stream));
+    ctx->c_d2h += (int64_t)(cells * sizeof(int32_t));
+    return VPCA_OK;
+}
+
+int vpca_project_pca(vpca_ctx* ctx, int32_t k, double* out) {
+    if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (ctx->proj_k == 0) return fail(ctx, VPCA_ERR_STATE, "call vpca_compute_pca first");
+    if (k < 1 || k > ctx->proj_k)
+        return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_project_pca: k=%d outside [1, %d] (the k of the last vpca_compute_pca)", k,
+                    ctx->proj_k);
+    if (ctx->n_proj == 0) return VPCA_OK;
+    if (out == nullptr) return fail(ctx, VPCA_ERR_BAD_ARG, "out is NULL");
+    CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
+    const int m = ctx->n_proj, kmax = std::max(ctx->num_pc, 16);
+    const size_t part = (size_t)proj_chunks(ctx->n) * m * kmax;
+    if (ctx->d_proj == nullptr) {
+        cudaError_t e = cudaMalloc(&ctx->d_proj, ((size_t)m + part + (size_t)m * kmax) * sizeof(double));
+        if (e != cudaSuccess) {
+            ctx->d_proj = nullptr;
+            return fail(ctx, VPCA_ERR_NOMEM, "projection workspace: %s", cudaGetErrorString(e));
+        }
+    }
+    double* d_rowmean = ctx->d_proj;
+    double* d_part = d_rowmean + m;
+    double* d_y = d_part + part;
+    CUDA_OK(ctx, eig_project(ctx->eig, ctx->d_S + (size_t)ctx->n * ctx->n, m, k, d_rowmean, d_part, d_y, ctx->stream));
+    ctx->c_launches += 3;
+    CUDA_OK(ctx, cudaMemcpyAsync(out, d_y, (size_t)m * k * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_OK(ctx, cudaStreamSynchronize(ctx->stream));
+    ctx->c_d2h += (int64_t)m * k * 8;
+    return VPCA_OK;
+}
+
+int vpca_debug_projection_tiles(int32_t n_fit, int32_t n_total, int32_t cta_group, int32_t mxf4, int32_t* out,
+                                int32_t max_tiles) {
+    if (n_fit < 1 || n_total < n_fit || max_tiles < 0 || (out == nullptr && max_tiles > 0))
+        return fail(nullptr, VPCA_ERR_BAD_ARG, "vpca_debug_projection_tiles: bad argument");
+    return gram_debug_projection_tiles(n_fit, n_total, cta_group, mxf4 != 0, out, max_tiles);
 }
 
 int vpca_get_centered(vpca_ctx* ctx, double* out) {
@@ -1258,7 +1369,7 @@ int vpca_synth_dense_device(vpca_ctx* ctx, uint64_t seed, int64_t v0, int64_t nv
     if (mode == 1 && ctx->max_mult < 2)
         return fail(ctx, VPCA_ERR_BAD_ARG, "dosage mode needs max_multiplicity >= 2");
     CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
-    cudaError_t e = synth_dense(seed, ctx->n, v0, nv, mode, ctx->elem_bits, d_x, ld, 0, ctx->stream);
+    cudaError_t e = synth_dense(seed, ctx->rows(), v0, nv, mode, ctx->elem_bits, d_x, ld, 0, ctx->stream);
     if (e != cudaSuccess) return fail(ctx, VPCA_ERR_CUDA, "synthetic generator: %s", cudaGetErrorString(e));
     ctx->c_launches += 2 * ((nv + (1 << 22) - 1) >> 22);
     return VPCA_OK;
@@ -1289,6 +1400,7 @@ int vpca_get_stats(vpca_ctx* ctx, vpca_stats* out) {
 int vpca_gram_export_ipc(vpca_ctx* ctx, void* handle64) {
     if (ctx == nullptr || handle64 == nullptr) return fail(ctx, VPCA_ERR_BAD_ARG, "NULL argument");
     std::lock_guard<std::mutex> lk(ctx->mu);
+    if (ctx->n_proj > 0) return fail(ctx, VPCA_ERR_UNSUPPORTED, "projecting contexts reduce through vpca_gram_device_ptr");
     if (!ctx->own_S) return fail(ctx, VPCA_ERR_STATE, "the peer-reduce mode needs a library-owned Gram (vpca_config.d_gram == NULL)");
     if (ctx->band_rows != ctx->n) return fail(ctx, VPCA_ERR_STATE, "band-only Grams are shared with vpca_gram_set_peers_local");
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "cudaIpcMemHandle_t is 64 bytes");
@@ -1303,6 +1415,7 @@ int vpca_gram_set_peers(vpca_ctx* ctx, const void* handles, int32_t world, int32
     if (ctx == nullptr || handles == nullptr || world < 1 || world > 16 || rank < 0 || rank >= world)
         return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_gram_set_peers: bad argument (world <= 16)");
     std::lock_guard<std::mutex> lk(ctx->mu);
+    if (ctx->n_proj > 0) return fail(ctx, VPCA_ERR_UNSUPPORTED, "projecting contexts reduce through vpca_gram_device_ptr");
     if (!ctx->own_S) return fail(ctx, VPCA_ERR_STATE, "the peer-reduce mode needs a library-owned Gram");
     if (ctx->plan.num_peers != 0) return fail(ctx, VPCA_ERR_STATE, "peers already set");
     CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
@@ -1342,6 +1455,8 @@ int vpca_gram_set_peers_local(vpca_ctx* const* ctxs, int32_t world) {
     if (ctxs == nullptr || world < 1 || world > 16) return fail(nullptr, VPCA_ERR_BAD_ARG, "vpca_gram_set_peers_local: world must be in [1, 16]");
     for (int r = 0; r < world; ++r) {
         if (ctxs[r] == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctxs[%d] is NULL", r);
+        if (ctxs[r]->n_proj > 0)
+            return fail(ctxs[r], VPCA_ERR_UNSUPPORTED, "projecting contexts reduce through vpca_gram_device_ptr");
         if (!ctxs[r]->own_S) return fail(ctxs[r], VPCA_ERR_STATE, "the peer-reduce mode needs a library-owned Gram");
         if (ctxs[r]->n != ctxs[0]->n) return fail(ctxs[r], VPCA_ERR_BAD_ARG, "all contexts must have the same n_samples");
         if (ctxs[r]->plan.num_peers != 0) return fail(ctxs[r], VPCA_ERR_STATE, "peers already set");

@@ -45,7 +45,8 @@ struct GramPlan {
                               // B200, 2504 x 1M int8: 0.5 settles at 1.61 ms within three launches, 0.7 and 1.0 hover at 1.70)
     bool adaptive = true;     // VPCA_ADAPTIVE=0 keeps the stream-K split equal instead of speed-weighted
     double* d_cum = nullptr;  // cumulative worker shares (workers + 1 doubles) + update counter
-    int cum_workers = 0, cum_tiles = 0, cum_kbw = 0, cum_for_n = 0, cum_dev = 0, cum_elem = 0;   // what the split in d_cum was made for
+    int cum_workers = 0, cum_tiles = 0, cum_kbw = 0, cum_for_n = 0, cum_for_rows = 0, cum_dev = 0, cum_elem = 0;   // what the
+                                                                                    // split in d_cum was made for
     // fused multi-GPU reduction: Gram buffers / barrier flags of all ranks, peer-mapped through CUDA IPC
     int num_peers = 0, peer_rank = 0, peer_epoch = 0;
     int32_t* peer_S[16] = {};     // Gram of rank d as seen from this device: the address of row 0 (for a rank that stores
@@ -65,14 +66,15 @@ int gram_read_profile(GramPlan& plan, long long* out, int max_ctas);
 // S(lower triangle, row >= col) += X X^T for the nv variants of a dense sample-major tile.
 //   d_x : device, element (s, v) at index s * ld + v; elem_bits 8 (int8), 16 (bf16) or 4 (packed e2m1: two cells per
 //         byte, ld % 128 == 0 and zero cells up to the next multiple of 128 variants)
-//   d_S : device int32 n x n row-major
+//   d_S : device int32 n_rows x n row-major (pitch n): rows [0, n) the fitted Gram, rows [n, n_rows) the cross block of
+//         the projected samples (n_rows == n: a plain context).  Only cells with row >= col < n are written.
 // Returns cudaSuccess or the first CUDA error; never synchronises.
 // panel > 0: the tile is stored as ceil(nv / panel) consecutive panels of `panel` variants, each panel n rows of
 // `panel` cells (cell (s, v) at (v / panel) * n * panel + s * panel + v % panel, zero cells after nv in the last
 // panel); `ld` is ignored.  Keeps the pages touched per L2 window few (a row-major tile with a multi-MB pitch puts
 // every sample row on its own 2 MB page and thrashes the TLBs).
-cudaError_t gram_accumulate(GramPlan& plan, const void* d_x, int elem_bits, int n, int64_t nv, int64_t ld, int64_t panel,
-                            int32_t* d_S, cudaStream_t stream, std::string* err);
+cudaError_t gram_accumulate(GramPlan& plan, const void* d_x, int elem_bits, int n, int n_rows, int64_t nv, int64_t ld,
+                            int64_t panel, int32_t* d_S, cudaStream_t stream, std::string* err);
 cudaError_t gram_symmetrize(int32_t* d_S, int n, cudaStream_t stream);
 cudaError_t gram_add(int32_t* d_dst, const int32_t* d_src, int64_t count, cudaStream_t stream);
 cudaError_t gram_add_peers(GramPlan& plan, const int32_t* d_src, int64_t count, cudaStream_t stream);
@@ -84,6 +86,7 @@ cudaError_t encode_preload_kernels();
 void gram_plan_free(GramPlan& plan);
 int gram_debug_max_clusters(int cluster_size);
 int gram_debug_band_tiles(int n, int cta_group, int row_lo, int row_hi, int32_t* out, int max_tiles);
+int gram_debug_projection_tiles(int n_fit, int n_total, int cta_group, bool mxf4, int32_t* out, int max_tiles);
 int gram_debug_tiles(int n, int cta_group, int exact, int32_t* out, int max_tiles);
 int gram_debug_plan(const int32_t* tiles8, int num_tiles, int workers, int kbw, int32_t* out, int max_pieces);
 int gram_debug_repair(const int32_t* tiles8, int num_tiles, int workers, int kbw, int col_limit, double* cum, int32_t* out,
@@ -91,16 +94,16 @@ int gram_debug_repair(const int32_t* tiles8, int num_tiles, int workers, int kbw
 
 // ---- encode (encode.cu) ------------------------------------------------------------------------
 // CSR rows [0, nv) (d_off has nv+1 entries; entry e of row v is d_idx[d_off[v] - base + ...]) -> dense
-// sample-major tile, zero-filled first.  d_flags[0] is OR-ed with 1 on an out-of-range index and 2 on a
-// multiplicity overflow.
+// sample-major tile of n rows, zero-filled first.  d_flags[0] is OR-ed with 1 on an index outside [0, n) and 2 on a
+// multiplicity overflow.  d_rows (n entries, may be nullptr = identity): the tile row of input sample s.
 cudaError_t encode_calls(const int64_t* d_off, int64_t base, const void* d_idx, int idx_bytes, int64_t nv, int n,
-                         int elem_bits, int max_mult, void* d_x, int64_t ld, int64_t panel, int* d_flags,
-                         cudaStream_t stream);   // idx_bytes: 4 (int32) or 2 (uint16)
+                         int elem_bits, int max_mult, void* d_x, int64_t ld, int64_t panel, const int32_t* d_rows,
+                         int* d_flags, cudaStream_t stream);   // idx_bytes: 4 (int32) or 2 (uint16)
 
 // Packed rows (`stride` bytes apart) -> dense cells (binary carriers).  code 0: one N-bit bitmap per variant, LSB
 // first; code 1 / 2: PLINK .bed rows (2 bits per sample), carriers of A1 / of A2.
 cudaError_t encode_bits(const uint8_t* d_bits, int64_t stride, int64_t nv, int n, int elem_bits, void* d_x, int64_t ld,
-                        int64_t panel, int code, cudaStream_t stream);
+                        int64_t panel, int code, const int32_t* d_rows, cudaStream_t stream);
 
 // ---- multi-dataset keying: variant keys, join, merge (join.cu) ---------------------------------------------
 struct JoinWork {
@@ -146,6 +149,7 @@ struct EigWork {
     double* d_off = nullptr;   // n
     double* d_tau = nullptr;   // n
     double* d_scal = nullptr;  // small scalar scratch
+    double* d_mm = nullptr;    // matrixMean of the last center_gram (d_scal[0] does not survive the solvers)
     double* d_evals = nullptr; // k
     double* d_evecs = nullptr; // n x k (column-major)
     double* d_lu = nullptr;    // 8 n scratch for inverse iteration
@@ -177,6 +181,12 @@ void eig_free(EigWork& w);
 cudaError_t center_gram(EigWork& w, const int32_t* d_S, cudaStream_t stream, bool materialise);
 cudaError_t center_matrix(EigWork& w, cudaStream_t stream);
 cudaError_t eig_topk(EigWork& w, int k, cudaStream_t stream, int64_t* launches);
+// Projection of m cross rows d_X (m x w.n int32, pitch w.n) onto the first k vectors of the last eig_topk, with the row
+// sums and matrixMean of the last center_gram: d_y (m x k, column-major).  Scratch: d_rowmean (m), d_part
+// (proj_chunks(w.n) * m * k).  Three launches.
+int proj_chunks(int n);
+cudaError_t eig_project(const EigWork& w, const int32_t* d_X, int m, int k, double* d_rowmean, double* d_part, double* d_y,
+                        cudaStream_t stream);
 
 // ---- synthetic generator (synth.cu) ----------------------------------------------------------------
 cudaError_t synth_dense(uint64_t seed, int n, int64_t v0, int64_t nv, int mode, int elem_bits, void* d_x,

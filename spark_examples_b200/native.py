@@ -50,6 +50,7 @@ EXPORTED_SYMBOLS = (
     "vpca_pool_accumulate_calls", "vpca_pool_accumulate_calls_u16", "vpca_pool_accumulate_bits", "vpca_pool_accumulate_bed",
     "vpca_pool_commit", "vpca_pool_abort", "vpca_pool_reduce_and_finalize", "vpca_pool_get_gram", "vpca_pool_compute_pca",
     "vpca_pool_get_stats", "vpca_debug_tiles", "vpca_debug_plan",
+    "vpca_create_projecting", "vpca_get_cross_gram", "vpca_project_pca", "vpca_debug_projection_tiles",
 )
 
 
@@ -81,6 +82,14 @@ class VpcaConfig(ctypes.Structure):
         ("d_gram", ctypes.c_void_p),
         ("gram_band_row0", ctypes.c_int32),
         ("gram_band_rows", ctypes.c_int32),
+    ]
+
+
+class VpcaProjection(ctypes.Structure):
+    _fields_ = [
+        ("struct_size", ctypes.c_uint32),
+        ("n_projected", ctypes.c_int32),
+        ("sample_rows", ctypes.POINTER(ctypes.c_int32)),
     ]
 
 
@@ -248,6 +257,14 @@ def load_library() -> ctypes.CDLL:
     L.vpca_gram_gather.argtypes = [vp]
     L.vpca_debug_gram_profile.restype = ctypes.c_int
     L.vpca_debug_gram_profile.argtypes = [vp, vp, i32]
+    L.vpca_create_projecting.restype = ctypes.c_int
+    L.vpca_create_projecting.argtypes = [ctypes.POINTER(VpcaConfig), ctypes.POINTER(VpcaProjection), ctypes.POINTER(vp)]
+    L.vpca_get_cross_gram.restype = ctypes.c_int
+    L.vpca_get_cross_gram.argtypes = [vp, vp]
+    L.vpca_project_pca.restype = ctypes.c_int
+    L.vpca_project_pca.argtypes = [vp, i32, vp]
+    L.vpca_debug_projection_tiles.restype = ctypes.c_int
+    L.vpca_debug_projection_tiles.argtypes = [i32, i32, i32, i32, vp, i32]
     _lib = L
     return L
 
@@ -262,9 +279,14 @@ class NativePca:
     def __init__(self, n_samples: int, device: int = 0, dtype: int = DTYPE_I8, num_pc: int = 2,
                  max_multiplicity: int = 2, partitions_in_flight: int = 4, chunk_variants: int = 0,
                  chunk_nnz: int = 0, stream: int = 0, d_gram: int = 0, staging_lanes: int = 0,
-                 gram_band: Optional[Tuple[int, int]] = None):
+                 gram_band: Optional[Tuple[int, int]] = None, n_projected: int = 0, sample_rows=None):
+        """n_projected > 0 (or a sample_rows map): a projecting context (vpca_create_projecting) -- n_samples fitted
+        samples plus n_projected ones placed on the fitted PCs by projectPca.  sample_rows: input sample position ->
+        row of the context (fitted rows first), None = the last n_projected inputs are the projected ones."""
         self._lib = load_library()
         self.n = int(n_samples)
+        self.n_projected = int(n_projected)
+        self.rows = self.n + self.n_projected   # rows of the genotype tiles and of the Gram buffer
         self.dtype = int(dtype)
         self.elem_bits = {DTYPE_I8: 8, DTYPE_BF16: 16, DTYPE_E2M1: 4}[self.dtype]
         self.elem_bytes = self.elem_bits / 8
@@ -274,7 +296,17 @@ class NativePca:
                          partitions_in_flight, staging_lanes, chunk_variants, chunk_nnz, stream or None, d_gram or None,
                          row0, rows)
         handle = ctypes.c_void_p()
-        rc = self._lib.vpca_create(ctypes.byref(cfg), ctypes.byref(handle))
+        if self.n_projected > 0 or sample_rows is not None:
+            rows_map = None
+            if sample_rows is not None:
+                rows_map = np.ascontiguousarray(sample_rows, dtype=np.int32)
+                if rows_map.shape != (self.rows,):
+                    raise VpcaError(VPCA_ERR_BAD_ARG, f"sample_rows must have n_samples + n_projected = {self.rows} entries")
+            proj = VpcaProjection(ctypes.sizeof(VpcaProjection), self.n_projected,
+                                  rows_map.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)) if rows_map is not None else None)
+            rc = self._lib.vpca_create_projecting(ctypes.byref(cfg), ctypes.byref(proj), ctypes.byref(handle))
+        else:
+            rc = self._lib.vpca_create(ctypes.byref(cfg), ctypes.byref(handle))
         self._h = handle if rc == VPCA_OK else None
         if rc != VPCA_OK:
             self._raise(rc, None)
@@ -325,11 +357,11 @@ class NativePca:
         nv = len(off) - 1
         if self.elem_bits == 4:                      # packed: (n, ld / 2) bytes, ld a multiple of 128 cells
             ld = max(128, ((nv + 127) // 128) * 128)
-            out = np.zeros((self.n, ld // 2), dtype=np.uint8)
+            out = np.zeros((self.rows, ld // 2), dtype=np.uint8)
             self._check(self._lib.vpca_encode_calls(self._h, _host_ptr(off), _host_ptr(idx) if len(idx) else None, nv,
                                                     _host_ptr(out), ld))
             return out
-        out = np.zeros((self.n, max(nv, 1)), dtype=np.int8 if self.elem_bits == 8 else np.uint16)
+        out = np.zeros((self.rows, max(nv, 1)), dtype=np.int8 if self.elem_bits == 8 else np.uint16)
         self._check(self._lib.vpca_encode_calls(self._h, _host_ptr(off), _host_ptr(idx) if len(idx) else None, nv,
                                                 _host_ptr(out), out.shape[1]))
         return out[:, :nv]
@@ -439,15 +471,15 @@ class NativePca:
         (n, ld / 2) with ld % 128 == 0, `nv` valid cells per row and zero cells after them."""
         x = np.asarray(x)
         if self.elem_bits == 4:
-            if x.dtype != np.uint8 or x.ndim != 2 or x.shape[0] != self.n or (x.shape[1] * 2) % 128:
-                raise VpcaError(VPCA_ERR_BAD_ARG, f"packed tile must be ({self.n}, ld/2) uint8 with ld % 128 == 0")
+            if x.dtype != np.uint8 or x.ndim != 2 or x.shape[0] != self.rows or (x.shape[1] * 2) % 128:
+                raise VpcaError(VPCA_ERR_BAD_ARG, f"packed tile must be ({self.rows}, ld/2) uint8 with ld % 128 == 0")
             x = np.ascontiguousarray(x)
             ld = x.shape[1] * 2
             self._check(self._lib.vpca_accumulate_dense(self._h, _host_ptr(x), ld if nv is None else int(nv), ld, 0))
             return
         want = np.int8 if self.elem_bits == 8 else np.uint16
-        if x.dtype != want or x.ndim != 2 or x.shape[0] != self.n:
-            raise VpcaError(VPCA_ERR_BAD_ARG, f"dense tile must be ({self.n}, nv) {np.dtype(want).name}")
+        if x.dtype != want or x.ndim != 2 or x.shape[0] != self.rows:
+            raise VpcaError(VPCA_ERR_BAD_ARG, f"dense tile must be ({self.rows}, nv) {np.dtype(want).name}")
         if not x.flags.c_contiguous:
             x = np.ascontiguousarray(x)
         self._check(self._lib.vpca_accumulate_dense(self._h, _host_ptr(x), x.shape[1], x.shape[1], 0))
@@ -465,7 +497,7 @@ class NativePca:
 
     def panelBytes(self, nv: int, panel_variants: int) -> int:
         npanels = (int(nv) + panel_variants - 1) // panel_variants
-        return npanels * self.n * panel_variants * self.elem_bits // 8
+        return npanels * self.rows * panel_variants * self.elem_bits // 8
 
     def gramDevicePtr(self) -> int:
         p = ctypes.c_void_p()
@@ -501,8 +533,9 @@ class NativePca:
 
     def partialGram(self, with_count: bool = False):
         """The accumulated (not yet finalized) Gram: lower triangle meaningful.  Checkpoint payload (with_count: also
-        the number of variants the counts stand for, which a resume hands back to loadPartialGram)."""
-        out = np.empty((self.n, self.n), dtype=np.int32)
+        the number of variants the counts stand for, which a resume hands back to loadPartialGram).  Projecting
+        contexts: (n + n_projected, n), the cross block below the fitted Gram."""
+        out = np.empty((self.rows, self.n), dtype=np.int32)
         nv = ctypes.c_int64(0)
         self._check(self._lib.vpca_get_partial_gram(self._h, _host_ptr(out), ctypes.byref(nv)))
         return (out, int(nv.value)) if with_count else out
@@ -511,8 +544,8 @@ class NativePca:
         """Restore a checkpointed partial Gram; accumulation continues on top of it (and keeps counting against the
         int32 bound of a similarity count from `variants_in_gram`)."""
         g = np.ascontiguousarray(gram, dtype=np.int32)
-        if g.shape != (self.n, self.n):
-            raise VpcaError(VPCA_ERR_BAD_ARG, "gram must be (n, n)")
+        if g.shape != (self.rows, self.n):
+            raise VpcaError(VPCA_ERR_BAD_ARG, "gram must be (n + n_projected, n)")
         self._check(self._lib.vpca_load_partial_gram(self._h, _host_ptr(g), int(variants_in_gram)))
 
     def variantCount(self) -> int:
@@ -544,6 +577,18 @@ class NativePca:
         nz = ctypes.c_int32(0)
         self._check(self._lib.vpca_compute_pca(self._h, int(k), _host_ptr(flat), _host_ptr(evals), ctypes.byref(nz)))
         return flat.reshape(k, self.n).T.copy(), evals, int(nz.value)
+
+    def crossGram(self) -> np.ndarray:
+        """(n_projected, n) int32: variants each projected sample shares with each fitted one (after finalizeGram)."""
+        out = np.empty((self.n_projected, self.n), dtype=np.int32)
+        self._check(self._lib.vpca_get_cross_gram(self._h, _host_ptr(out)))
+        return out
+
+    def projectPca(self, k: int = 2) -> np.ndarray:
+        """(n_projected, k) float64: coordinates of the projected samples on the first k PCs of the last computePca."""
+        flat = np.empty(max(self.n_projected * k, 1), dtype=np.float64)
+        self._check(self._lib.vpca_project_pca(self._h, int(k), _host_ptr(flat)))
+        return flat[:self.n_projected * k].reshape(k, self.n_projected).T.copy()
 
     def getCentered(self) -> np.ndarray:
         out = np.empty((self.n, self.n), dtype=np.float64)
@@ -595,6 +640,17 @@ def debugPlan(tiles: np.ndarray, workers: int, kb_window: int) -> np.ndarray:
     if cnt < 0:
         raise VpcaError(VPCA_ERR_STATE, L.vpca_last_error(None).decode("utf-8", "replace"))
     return out[:cnt]
+
+
+def debugProjectionTiles(n_fit: int, n_total: int, cta_group: int, mxf4: bool) -> np.ndarray:
+    """Tiles of a projecting context (vpca_debug_projection_tiles), (tiles, 8) int32 like debugTiles."""
+    L = load_library()
+    cnt = L.vpca_debug_projection_tiles(int(n_fit), int(n_total), int(cta_group), 1 if mxf4 else 0, None, 0)
+    if cnt < 0:
+        raise VpcaError(cnt, L.vpca_last_error(None).decode("utf-8", "replace"))
+    out = np.zeros((cnt, 8), dtype=np.int32)
+    L.vpca_debug_projection_tiles(int(n_fit), int(n_total), int(cta_group), 1 if mxf4 else 0, _host_ptr(out), cnt)
+    return out
 
 
 def debugBandTiles(n_samples: int, cta_group: int, row0: int, rows: int) -> np.ndarray:

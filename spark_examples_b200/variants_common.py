@@ -7,6 +7,10 @@ rows 11-12); what the hot path needs from it is kept: `indexes` (callset id -> d
 order, :44-45), `names` (:46-47) and `data`, a list of datasets of `Variant` records split in partitions.
 Sources here: `--input-path` (a JSON-lines stand-in for the saved object file of :53-55), `--synthetic N,V[,seed]`
 (device generator, DESIGN.md) or records handed over in memory.
+
+`--projected-callsets FILE` (additive) names callsets that are placed on the principal components of the others
+instead of being fitted: `indexes` keeps source order, and `sample_rows` maps every source index to its row of the
+GPU context -- fitted callsets first, then the projected ones, each in source order.
 """
 from __future__ import annotations
 
@@ -130,6 +134,7 @@ class VariantsCommon:
                 "The Google Genomics API the reference streams from (VariantsCommon.scala:38-66) is retired; "
                 "give --vcf-path FILE.vcf[.gz][,...], --bed-path PLINK_PREFIX, --calls-parquet-path FILE, --input-path FILE.jsonl "
                 "or --synthetic N,V[,seed]")
+        self._set_projection(conf)
         print(f"Matrix size: {len(self.indexes)}.")                 # :48
 
     def _set_callsets(self, callsets: Sequence[Tuple[str, str]]):
@@ -139,9 +144,57 @@ class VariantsCommon:
             raise ValueError("duplicate callset id")
         self.names: Dict[str, str] = {c[0]: c[1] for c in callsets}              # :46-47
 
+    def _set_projection(self, conf: PcaConf):
+        """`n_projected` and `sample_rows` (source index -> context row) from --projected-callsets."""
+        n = len(self.indexes)
+        self.n_projected = 0
+        self.sample_rows = np.arange(n, dtype=np.int32)
+        if not conf.projectedCallsets.isDefined:
+            return
+        self.n_projected, self.sample_rows = projection_rows(self.names, self.indexes,
+                                                             read_projected_names(conf.projectedCallsets()))
+        if conf.synthetic.isDefined and not np.array_equal(self.sample_rows, np.arange(n, dtype=np.int32)):
+            raise ValueError("--synthetic generates its cohort in row order: only the trailing callsets can be projected")
+
+    @property
+    def n_fitted(self) -> int:
+        return len(self.indexes) - self.n_projected
+
     def reportIoStats(self):                                        # :68-73
         if self.ioStats is not None:
             print(self.ioStats)
+
+
+def read_projected_names(path: str) -> List[str]:
+    """One callset name per line (the first output column); blank lines are ignored."""
+    with open(path, "r", encoding="utf-8") as fh:
+        return [ln.strip() for ln in fh if ln.strip()]
+
+
+def projection_rows(names: Dict[str, str], indexes: Dict[str, int], projected: Sequence[str]) -> Tuple[int, np.ndarray]:
+    """(M, sample_rows): the callsets whose name is listed are projected.  sample_rows[source index] = row of the GPU
+    context: fitted callsets get rows 0..N-1 and projected ones N..N+M-1, each group in source order.  A name that
+    matches no callset or several, and a list that leaves nothing to fit, are errors."""
+    by_name: Dict[str, List[str]] = {}
+    for cid, name in names.items():
+        by_name.setdefault(name, []).append(cid)
+    chosen = set()
+    for name in projected:
+        ids = by_name.get(name, [])
+        if not ids:
+            raise ValueError(f"--projected-callsets: no callset is named {name!r}")
+        if len(ids) > 1:
+            raise ValueError(f"--projected-callsets: {len(ids)} callsets are named {name!r}")
+        chosen.add(ids[0])
+    total = len(indexes)
+    if len(chosen) >= total:
+        raise ValueError("--projected-callsets lists every callset: nothing is left to fit")
+    order = sorted(indexes.items(), key=lambda kv: kv[1])
+    fitted = [i for cid, i in order if cid not in chosen]
+    proj = [i for cid, i in order if cid in chosen]
+    rows = np.empty(total, dtype=np.int32)
+    rows[np.asarray(fitted + proj, dtype=np.int64)] = np.arange(total, dtype=np.int32)
+    return len(proj), rows
 
 
 def _chunk(items: List[object], size: int) -> List[List[object]]:

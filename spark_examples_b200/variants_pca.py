@@ -273,7 +273,7 @@ class VariantsPcaDriver:
     def getSimilarityMatrix(self, callsets: CallsRdd) -> SimilarityMatrix:
         """S = sum over variants of x x^T on the GPU: every partition is one `mapPartitions` task (encode + tcgen05
         Gram into a private staging Gram, committed on success); `reduceByKey(_ + _)` across ranks is one all-reduce."""
-        nat = self._native(callsets.n_samples)
+        nat = self._native(self.common.n_fitted)
         nat.reset()
         done = self._load_checkpoint(nat, callsets)
         for pid, part in enumerate(callsets.partitions):
@@ -307,7 +307,7 @@ class VariantsPcaDriver:
                                        "int32 similarity count")
             vdist.allreduce_gram(self._gram_tensor)            # VariantsPca.scala:190
         nat.finalizeGram()
-        return SimilarityMatrix(nat, callsets.n_samples)
+        return SimilarityMatrix(nat, self.common.n_fitted)
 
     def getSimilarityMatrixStream(self, calls: CallsRdd) -> SimilarityMatrix:
         """VariantsPca.scala:262-279 yields the same matrix (its sparse-row quirk is not reproduced, SURVEY.md 2 row 3);
@@ -319,7 +319,7 @@ class VariantsPcaDriver:
         """`matrixEntries`: what getSimilarityMatrix returned (stays on the GPU), or -- the reference's signature,
         `RDD[((Int, Int), Int)]` (:198) -- any iterable of ((row, col), count) records, which are loaded into the GPU
         (absent keys count 0, like the rows `:216-221` never see)."""
-        rowCount = len(self.common.indexes)
+        rowCount = self.common.n_fitted
         numPc = self.conf.numPc()
         if numPc < 2:
             # the reference reads array(i + pca.numRows) (:230) and fails for numPc = 1
@@ -327,6 +327,8 @@ class VariantsPcaDriver:
         if isinstance(matrixEntries, SimilarityMatrix):
             nat = matrixEntries._nat
         else:
+            if self.common.n_projected:
+                raise ValueError("--projected-callsets needs the similarity matrix getSimilarityMatrix computed")
             S = np.zeros((rowCount, rowCount), np.int32)
             for (i, j), v in matrixEntries:
                 S[i, j] = v                                                      # IndexError like Breeze at :216
@@ -336,11 +338,24 @@ class VariantsPcaDriver:
         print(f"Non zero rows in matrix: {nonZeroRows} / {rowCount}.")           # :208
         self.eigenvalues = evals
         self.components = vecs                                                   # all numPc columns (Python twin prints them)
-        reverse = {i: cid for cid, i in self.common.indexes.items()}             # :228
+        self._pca_nat = nat
+        reverse = self._row_to_callset()                                         # :228
         return [(reverse[i], float(vecs[i, 0]), float(vecs[i, 1])) for i in range(rowCount)]   # :229-230
 
+    def projectPca(self) -> List[Tuple[str, float, float]]:
+        """The callsets of --projected-callsets on the first two PCs of the last computePca: (callsetId, pc1, pc2).  Not
+        in the reference: Gower's add-a-point formula on the cross counts, centred with the fitted statistics
+        (include/vpca.h, DESIGN.md 3.6); projected coordinates are not corrected for their shrinkage towards 0."""
+        y = self._pca_nat.projectPca(self.conf.numPc())
+        reverse, n = self._row_to_callset(), self.common.n_fitted
+        return [(reverse[n + p], float(y[p, 0]), float(y[p, 1])) for p in range(self.common.n_projected)]
+
+    def _row_to_callset(self) -> Dict[int, str]:
+        rows = self.common.sample_rows
+        return {int(rows[i]): cid for cid, i in self.common.indexes.items()}
+
     # -- VariantsPca.scala:233-246 ----------------------------------------------------------------------------------
-    def emitResult(self, result: Sequence[Tuple[str, float, float]], out=None):
+    def emitResult(self, result: Sequence[Tuple[str, float, float]], out=None, suffix: str = "-pca.tsv"):
         out = out or sys.stdout
         rows = []
         for callset_id, pc1, pc2 in result:
@@ -350,12 +365,19 @@ class VariantsPcaDriver:
             for name, pc1, pc2, dataset in sorted(rows, key=lambda t: t[0]):     # :238-239
                 out.write(f"{name}\t{dataset}\t{jdouble(pc1)}\t{jdouble(pc2)}\n")
             if self.conf.outputPath.isDefined:                                   # :241-245 (saveAsTextFile layout)
-                path = self.conf.outputPath() + "-pca.tsv"
+                path = self.conf.outputPath() + suffix
                 os.makedirs(path, exist_ok=True)
                 with open(os.path.join(path, "part-00000"), "w", encoding="utf-8") as fh:
                     for name, pc1, pc2, dataset in rows:
                         fh.write(f"{name}\t{jdouble(pc1)}\t{jdouble(pc2)}\t{dataset}\n")
                 open(os.path.join(path, "_SUCCESS"), "w").close()
+
+    def emitProjected(self, projected: Sequence[Tuple[str, float, float]], out=None):
+        """The projected samples after the fitted ones: a count line, then the rows in the layout of emitResult (and
+        `<output-path>-projected-pca.tsv`)."""
+        if self._rank == 0:
+            (out or sys.stdout).write(f"Projected samples: {len(projected)}.\n")
+        self.emitResult(projected, out, suffix="-projected-pca.tsv")
 
     def reportIoStats(self):                                                     # :281
         self.common.reportIoStats()
@@ -383,14 +405,19 @@ class VariantsPcaDriver:
                 torch.cuda.set_device(device)
                 self._torch_stream = torch.cuda.Stream(device=device)
                 torch.cuda.set_stream(self._torch_stream)
-                self._gram_tensor = torch.zeros((n, n), dtype=torch.int32, device=f"cuda:{device}")
+                # projecting runs: (N + M) x N, the cross block below the fitted Gram (one all-reduce moves both)
+                self._gram_tensor = torch.zeros((n + self.common.n_projected, n), dtype=torch.int32,
+                                                device=f"cuda:{device}")
                 stream, d_gram = self._torch_stream.cuda_stream, self._gram_tensor.data_ptr()
         except ImportError:
             pass
         if self._world > 1 and d_gram == 0:
             raise RuntimeError("multi-rank runs need torch with CUDA for the NCCL all-reduce")
+        proj = {}
+        if self.common.n_projected:
+            proj = dict(n_projected=self.common.n_projected, sample_rows=self.common.sample_rows)
         self._nat = native.NativePca(n, device=device, dtype=dtype, num_pc=max(2, self.conf.numPc()), stream=stream,
-                                     d_gram=d_gram)
+                                     d_gram=d_gram, **proj)
         return self._nat
 
     # -- checkpoint / resume (SURVEY 8f-2): the natural checkpoint of this job is the int32 Gram (25 MB at N = 2504)
@@ -409,6 +436,10 @@ class VariantsPcaDriver:
         ck = np.load(path)
         if int(ck["n_samples"]) != callsets.n_samples or int(ck["n_partitions"]) != len(callsets.partitions):
             raise ValueError(f"checkpoint {path} belongs to a different cohort / partitioning")
+        n_projected = int(ck["n_projected"]) if "n_projected" in ck.files else 0
+        rows = ck["sample_rows"] if "sample_rows" in ck.files else np.arange(callsets.n_samples, dtype=np.int32)
+        if n_projected != self.common.n_projected or not np.array_equal(rows, self.common.sample_rows):
+            raise ValueError(f"checkpoint {path} was written with other --projected-callsets")
         nat.loadPartialGram(ck["gram"], int(ck["variants"]))
         print(f"Resumed {len(ck['done'])} / {len(callsets.partitions)} partitions from {path}.")
         return set(int(p) for p in ck["done"])
@@ -419,8 +450,11 @@ class VariantsPcaDriver:
             return
         tmp = path + ".tmp.npz"
         gram, variants = nat.partialGram(with_count=True)
+        proj = {}
+        if self.common.n_projected:
+            proj = dict(n_projected=self.common.n_projected, sample_rows=self.common.sample_rows)
         np.savez(tmp, gram=gram, variants=variants, done=np.array(sorted(done), np.int64), n_samples=callsets.n_samples,
-                 n_partitions=len(callsets.partitions))
+                 n_partitions=len(callsets.partitions), **proj)
         os.replace(tmp, path)
 
     def _accumulate_synthetic(self, nat: native.NativePca, part: SyntheticSlice, panel: int = 8192):
@@ -490,6 +524,8 @@ def main(args: Optional[Sequence[str]] = None):
     simMatrix = driver.getSimilarityMatrix(callsRdd)
     result = driver.computePca(simMatrix)
     driver.emitResult(result)
+    if conf.projectedCallsets.isDefined:
+        driver.emitProjected(driver.projectPca())
     driver.reportIoStats()
     driver.stop()
     if int(os.environ.get("WORLD_SIZE", "1")) > 1:
