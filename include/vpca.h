@@ -273,6 +273,62 @@ int vpca_get_cross_gram(vpca_ctx* ctx, int32_t* out);
  * any vpca_compute_pca since the Gram last changed: VPCA_ERR_STATE.  Fixed reduction order: repeated calls are
  * bit-identical. */
 int vpca_project_pca(vpca_ctx* ctx, int32_t k, double* out);
+/* ---- saved model: project later without the panel genotypes ------------------------------------------------------
+ * Expanding X_pf = sum_v x_pv x_fv in the coordinate of vpca_project_pca gives the same number from per-variant
+ * quantities of the fitted panel (u_fc, lambda_c: the PCs of the last vpca_compute_pca; rs_f: the fitted row sums, :206):
+ *   loadings  L_vc = sum_f x_fv u_fc (FP64)   carriers  n_v = sum_f x_fv (exact)
+ *   col_sums  a_c = sum_f u_fc (~0)            rowsum_dots  b_c = sum_f (rs_f / N) u_fc
+ *   T_pc = sum_v x_pv L_vc,  r_p = sum_v x_pv n_v (= rs_p, exact),  y_pc = (((T_pc - (r_p / N) a_c) - b_c) + mean a_c) / lambda_c
+ * so {L, n, lambda, a, b, matrixMean} scores any cohort in one pass over its genotypes: no panel genotypes, no Gram and no
+ * eigensolve.  Not in the reference (it has no projection step, VariantsPca.scala:224-231): these numbers are not pinned
+ * by it.
+ *
+ * Fit side: a plain or projecting context after vpca_compute_pca; k <= the k of that call (else VPCA_ERR_BAD_ARG; before
+ * any vpca_compute_pca since the Gram last changed: VPCA_ERR_STATE).  The loadings calls take the same input as the
+ * accumulate calls (a second pass over the same rows), read the fitted rows 0..N-1 only, run on a lane like them and never
+ * touch the Gram or the partition staging.  Host outputs, one row per input variant in input order: loadings nv x k
+ * row-major, carriers nv.  The reduction over f has a fixed order that depends on f only, so a variant's loadings are
+ * bit-identical whatever route, chunking or call delivered it. */
+int vpca_pca_loadings_calls(vpca_ctx* ctx, int32_t k, const int64_t* offsets, const int32_t* sample_idx, int64_t nv,
+                            double* loadings, int32_t* carriers);
+int vpca_pca_loadings_bed(vpca_ctx* ctx, int32_t k, const uint8_t* rows, int64_t nv, int64_t stride_bytes,
+                          int32_t counted_allele, double* loadings, int32_t* carriers);
+int vpca_pca_loadings_panels(vpca_ctx* ctx, int32_t k, const void* d_x, int64_t nv, int64_t panel_variants,
+                             double* loadings, int32_t* carriers);
+/* The k eigenvalues, a (col_sums), b (rowsum_dots) and matrixMean of the last vpca_compute_pca (host outputs). */
+int vpca_pca_model_terms(vpca_ctx* ctx, int32_t k, double* eigenvalues, double* col_sums, double* rowsum_dots,
+                         double* matrix_mean);
+
+/* Scoring side.  A scoring context is a vpca_ctx whose cfg->n_samples are the M study samples; the model is copied to the
+ * device by the call.  cfg->d_gram and gram_band_rows must be unset: it allocates no Gram, and its Gram entry points
+ * (accumulate_*, finalize, get_gram / get_partial_gram / load_partial_gram / set_gram, compute_pca, project_pca, the
+ * peers) return VPCA_ERR_UNSUPPORTED.
+ *   vpca_score_calls / _bed: the input of vpca_accumulate_calls / _bed for the study samples, plus model_rows (nv): the
+ *     model row of each variant, -1 = not in the model (skipped); a row outside [-1, n_variants) gives
+ *     VPCA_ERR_INDEX_OUT_OF_RANGE.  partition_id >= 0: the scores stay private to the partition until vpca_commit (a
+ *     partition committed again replaces its earlier scores); vpca_abort discards them.  partition_id < 0: direct input.
+ *   vpca_score_panels: device-resident study cells in the panel layout of vpca_accumulate_panels (direct input).
+ *   vpca_score_project: out[p + c * M] = y_pc for c < k <= model->k (M x k column-major, like vpca_project_pca); the sum
+ *     runs over direct input first (in call order), then the committed partitions in ascending partition id, so the result
+ *     depends on how the input was cut into partitions and calls, never on thread timing or commit order.
+ *     *matched_variants (may be NULL): input variants with a model row.  VPCA_ERR_STATE while a partition is uncommitted. */
+typedef struct vpca_model {
+    uint32_t struct_size;          /* sizeof(vpca_model)                                                   */
+    int32_t n_fitted, k;           /* N of the fitted panel, columns of the model                          */
+    int64_t n_variants;            /* V (< 2^31)                                                           */
+    const double* loadings;        /* V x k row-major                                                      */
+    const int32_t* carriers;       /* V                                                                    */
+    const double* eigenvalues, *col_sums, *rowsum_dots;   /* k each                                    */
+    double matrix_mean;
+} vpca_model;
+int vpca_create_scoring(const vpca_config* cfg, const vpca_model* model, vpca_ctx** out);
+int vpca_score_calls(vpca_ctx* ctx, int64_t partition_id, const int64_t* offsets, const int32_t* sample_idx, int64_t nv,
+                     const int32_t* model_rows);
+int vpca_score_bed(vpca_ctx* ctx, int64_t partition_id, const uint8_t* rows, int64_t nv, int64_t stride_bytes,
+                   int32_t counted_allele, const int32_t* model_rows);
+int vpca_score_panels(vpca_ctx* ctx, const void* d_x, int64_t nv, int64_t panel_variants, const int32_t* model_rows);
+int vpca_score_project(vpca_ctx* ctx, int32_t k, double* out, int64_t* matched_variants /* may be NULL */);
+
 /* Host-only: the tiles (records of vpca_debug_tiles) of a projecting context with n_fit fitted and n_total - n_fit
  * projected samples -- A blocks over the n_fit columns of S, B rows over all n_total rows (row >= col); mxf4 != 0: the
  * 240-wide strips of kind::mxf4, else the 256-wide ones of int8 / bf16.  Returns the tile count (may exceed max_tiles). */

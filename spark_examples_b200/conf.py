@@ -114,4 +114,6 @@ class PcaConf(GenomicsConf):
             ("bedCountedAllele", str, "A1", False),       # which .bim allele is "variation": A1 (PLINK's minor) or A2
             ("projectedCallsets", str, None, False),      # file of callset names (one per line) placed on the PCs of the
                                                           # others instead of being fitted (VariantsPcaDriver.projectPca)
+            ("saveModel", str, None, False),              # after computePca: write the per-variant loadings model (model.py)
+            ("modelPath", str, None, False),              # score every callset against a saved model: no Gram, no eigensolve
         ]

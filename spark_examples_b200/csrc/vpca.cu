@@ -18,6 +18,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <map>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -52,6 +53,27 @@ struct vpca_ctx {
     double* d_proj = nullptr;      // projection scratch + result (eig_project)
     int rows() const { return n + n_proj; }                                        // rows of X
     size_t gram_cells() const { return (size_t)(band_rows + n_proj) * (size_t)n; }   // int32 cells of d_S
+    // scoring context (vpca_create_scoring): no Gram; the n samples are scored against a saved model that lives on the
+    // device.  An accumulator holds (T, r) of the model's k columns: n x k doubles, then n int64 (model.cu).
+    bool scoring = false;
+    int model_k = 0, model_nfit = 0;
+    int64_t model_nv = 0;
+    double* d_model_L = nullptr;      // model_nv x model_k
+    int32_t* d_model_n = nullptr;     // model_nv
+    double* d_model_terms = nullptr;  // lambda[k] | a[k] | b[k] | matrix mean
+    double* d_direct = nullptr;       // accumulator of direct input (partition_id < 0), in call order
+    int64_t direct_matched = 0;
+    std::mutex direct_mu;             // direct scoring calls add into d_direct one at a time
+    struct Scored {
+        double* d_acc = nullptr;
+        int64_t matched = 0;
+    };
+    std::map<int64_t, Scored> scored;   // committed partitions in ascending id
+    char* d_scratch = nullptr;          // model passes on the context's stream (panels routes, vpca_score_project)
+    int64_t cap_scratch = 0;
+    size_t slot_bytes() const {
+        return scoring ? (size_t)n * (model_k + 1) * sizeof(double) : (size_t)rows() * n * sizeof(int32_t);
+    }
     bool finalized = false;
     bool pca_done = false;
     GramPlan plan;        // schedule state of the launches on `stream` (device-resident input)
@@ -67,6 +89,7 @@ struct vpca_ctx {
         bool busy = false;             // a call of the owning task is in flight
         bool fresh = false;            // still to be zeroed by its first batch
         int64_t nv = 0;
+        int64_t matched = 0;           // scoring: variants with a model row
         cudaEvent_t ev_free = nullptr; // recorded after the commit that last read the slot
     };
     std::vector<Slot> slots;
@@ -85,6 +108,8 @@ struct vpca_ctx {
         int* d_flags = nullptr;
         int* h_flags = nullptr;
         GramPlan plan;
+        char* d_scratch = nullptr;   // loadings output / scoring model rows and partials (grow-only)
+        int64_t cap_scratch = 0;
         bool ready = false, busy = false;
     };
     std::vector<Lane> lanes;
@@ -130,6 +155,25 @@ int fail(vpca_ctx* ctx, int code, const char* fmt, ...) {
                         __LINE__);                                                                              \
     } while (0)
 
+// Entry points of the Gram on a scoring context (vpca_create_scoring), which has none.
+#define REFUSE_ON_SCORING(ctx)                                                                                  \
+    do {                                                                                                        \
+        if ((ctx)->scoring)                                                                                     \
+            return fail(ctx, VPCA_ERR_UNSUPPORTED, "%s: a scoring context has no Gram", __func__);              \
+    } while (0)
+
+template <typename T>
+static cudaError_t grow_buffer(T** p, int64_t* cap, int64_t need) {
+    if (need <= *cap && *p != nullptr) return cudaSuccess;
+    cudaFree(*p);
+    *p = nullptr;
+    *cap = 0;
+    const int64_t c = need + need / 4 + 1024;
+    cudaError_t e = cudaMalloc(p, (size_t)c * sizeof(T));
+    if (e == cudaSuccess) *cap = c;
+    return e;
+}
+
 // every similarity count is at most (#variants) * max_mult^2 and must stay a Java Int (VariantsPca.scala:185).
 // `extra` = variants about to be added on top of everything committed AND everything staged in uncommitted partitions.
 int check_overflow(vpca_ctx* ctx, int64_t extra) {
@@ -162,6 +206,9 @@ void free_lane(vpca_ctx::Lane& L) {
         }
     cudaFree(L.d_flags);
     L.d_flags = nullptr;
+    cudaFree(L.d_scratch);
+    L.d_scratch = nullptr;
+    L.cap_scratch = 0;
     if (L.h_flags) cudaFreeHost(L.h_flags);
     L.h_flags = nullptr;
     gram_plan_free(L.plan);
@@ -314,7 +361,7 @@ vpca_ctx::Slot* find_slot(vpca_ctx* ctx, int64_t pid, bool create, int* rc) {
     for (auto& s : ctx->slots)
         if (!s.used) {
             if (s.d_S == nullptr) {
-                cudaError_t e = cudaMalloc(&s.d_S, (size_t)ctx->rows() * ctx->n * sizeof(int32_t));
+                cudaError_t e = cudaMalloc(&s.d_S, ctx->slot_bytes());
                 if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.ev_free, cudaEventDisableTiming);
                 if (e != cudaSuccess) {
                     cudaFree(s.d_S);
@@ -328,6 +375,7 @@ vpca_ctx::Slot* find_slot(vpca_ctx* ctx, int64_t pid, bool create, int* rc) {
             s.busy = false;
             s.pid = pid;
             s.nv = 0;
+            s.matched = 0;
             return &s;
         }
     *rc = fail(ctx, VPCA_ERR_STATE, "more than %d partitions in flight; commit or abort one first",
@@ -340,15 +388,16 @@ vpca_ctx::Slot* find_slot(vpca_ctx* ctx, int64_t pid, bool create, int* rc) {
 struct CallScope {
     vpca_ctx* ctx;
     int64_t pid, nv;
+    int64_t matched = 0;   // scoring: variants of the call with a model row
     vpca_ctx::Slot* slot = nullptr;
-    int32_t* target = nullptr;
+    int32_t* target = nullptr;   // Gram / staging Gram; on a scoring context the (T, r) accumulator
     bool fresh = false;
     int begin() {
         std::lock_guard<std::mutex> lk(ctx->mu);
         if (ctx->finalized) return fail(ctx, VPCA_ERR_STATE, "Gram already finalized; call vpca_reset first");
-        int rc = check_overflow(ctx, nv);
+        int rc = ctx->scoring ? VPCA_OK : check_overflow(ctx, nv);   // scores accumulate in FP64 and int64
         if (rc != VPCA_OK) return rc;
-        target = ctx->d_S;
+        target = ctx->scoring ? reinterpret_cast<int32_t*>(ctx->d_direct) : ctx->d_S;
         if (pid >= 0) {
             slot = find_slot(ctx, pid, true, &rc);
             if (slot == nullptr) return rc;
@@ -374,6 +423,7 @@ struct CallScope {
             slot->busy = false;
             if (rc == VPCA_OK) {
                 slot->nv += nv;
+                slot->matched += matched;
             } else {
                 ctx->inflight_variants -= nv + slot->nv;
                 ctx->st.variants_accumulated -= slot->nv;
@@ -381,6 +431,7 @@ struct CallScope {
             }
         } else if (rc == VPCA_OK) {
             ctx->total_variants += nv;
+            ctx->direct_matched += matched;
         } else if (rc == VPCA_ERR_INDEX_OUT_OF_RANGE || rc == VPCA_ERR_OVERFLOW) {
             std::lock_guard<std::mutex> lk2(ctx->err_mu);
             ctx->err += " [direct accumulation: the Gram may hold a partial batch, call vpca_reset]";
@@ -395,7 +446,7 @@ struct CallScope {
 int prepare_slot(vpca_ctx* ctx, vpca_ctx::Lane& L, CallScope& sc) {
     if (sc.slot == nullptr || !sc.fresh) return VPCA_OK;
     CUDA_OK(ctx, cudaStreamWaitEvent(L.stream, sc.slot->ev_free, 0));
-    CUDA_OK(ctx, cudaMemsetAsync(sc.slot->d_S, 0, (size_t)ctx->rows() * ctx->n * sizeof(int32_t), L.stream));
+    CUDA_OK(ctx, cudaMemsetAsync(sc.slot->d_S, 0, ctx->slot_bytes(), L.stream));
     return VPCA_OK;
 }
 
@@ -410,9 +461,52 @@ void lane_gram_time(vpca_ctx* ctx, vpca_ctx::Lane& L) {
     }
 }
 
-// CSR rows -> encode -> (optionally) Gram, on lane L.  out_tile != nullptr: copy the encoded tile back instead.
+// What a chunk loop (process_calls, packed_chunks, the panels routes) does with each encoded chunk: the Gram launch,
+// the loadings of a saved model, or the scoring of a study against one (model.cu).
+struct ChunkSink {
+    enum Kind { GRAM, LOADINGS, SCORE } kind = GRAM;
+    int32_t* gram = nullptr;               // GRAM: the Gram or staging Gram the launch adds into
+    int k = 0;                             // LOADINGS / SCORE: columns
+    double* d_L = nullptr;                 // LOADINGS: device output of one chunk (nvc x k) ...
+    int32_t* d_cnt = nullptr;              // ... and its carriers
+    double* h_L = nullptr;                 // LOADINGS: host output of the call (nv x k) ...
+    int32_t* h_cnt = nullptr;              // ... and its carriers
+    const int32_t* d_mrows = nullptr;      // SCORE: model row of every variant of the call (device)
+    double* d_part = nullptr;              // SCORE: scratch of model_score
+    double* d_acc = nullptr;               // SCORE: the accumulator the chunk adds into
+    bool launched = false;                 // set once a Gram launch ran (lane timing)
+};
+
+// Consume variants [v, v + nvc) of the call, encoded in panel layout at d_x, on `stream`.
+int consume_chunk(vpca_ctx* ctx, GramPlan& plan, cudaStream_t stream, cudaEvent_t t0, cudaEvent_t t1, ChunkSink& sink,
+                  const void* d_x, int64_t v, int64_t nvc, int64_t panel) {
+    switch (sink.kind) {
+    case ChunkSink::GRAM: {
+        const int rc = launch_gram(ctx, plan, stream, t0, t1, d_x, nvc, panel, panel, sink.gram);
+        if (rc == VPCA_OK) sink.launched = true;
+        return rc;
+    }
+    case ChunkSink::LOADINGS:
+        CUDA_OK(ctx, model_loadings(d_x, ctx->elem_bits, nvc, panel, ctx->rows(), ctx->n, ctx->eig.d_evecs, sink.k, sink.d_L,
+                                    sink.d_cnt, stream));
+        CUDA_OK(ctx, cudaMemcpyAsync(sink.h_L + (size_t)v * sink.k, sink.d_L, (size_t)nvc * sink.k * sizeof(double),
+                                     cudaMemcpyDeviceToHost, stream));
+        CUDA_OK(ctx, cudaMemcpyAsync(sink.h_cnt + v, sink.d_cnt, (size_t)nvc * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+        ctx->c_launches += (sink.k + 7) / 8;
+        ctx->c_d2h += nvc * (sink.k * 8 + 4);
+        return VPCA_OK;
+    case ChunkSink::SCORE:
+        CUDA_OK(ctx, model_score(d_x, ctx->elem_bits, nvc, panel, ctx->rows(), sink.d_mrows + v, ctx->d_model_L, ctx->d_model_n,
+                                 sink.k, sink.d_part, sink.d_acc, stream));
+        ctx->c_launches += (sink.k + 7) / 8 + 1;
+        return VPCA_OK;
+    }
+    return fail(ctx, VPCA_ERR_BAD_ARG, "internal: unknown chunk consumer");
+}
+
+// CSR rows -> encode -> sink, on lane L.  out_tile != nullptr: copy the encoded tile back instead.
 int process_calls(vpca_ctx* ctx, vpca_ctx::Lane& L, const int64_t* offsets, const void* sample_idx, int idx_bytes,
-                  int64_t nv, int32_t* d_target, void* out_tile, int64_t out_ld) {
+                  int64_t nv, ChunkSink* sink, void* out_tile, int64_t out_ld) {
     const int bits = ctx->elem_bits;
     // validate the whole offsets array before anything is sized from it
     if (offsets[0] < 0) return fail(ctx, VPCA_ERR_BAD_ARG, "offsets[0] must be >= 0");
@@ -422,7 +516,6 @@ int process_calls(vpca_ctx* ctx, vpca_ctx::Lane& L, const int64_t* offsets, cons
     CUDA_OK(ctx, cudaMemsetAsync(L.d_flags, 0, sizeof(int), L.stream));
     int64_t v = 0;
     int chunk = 0;
-    bool launched = false;
     while (v < nv) {
         // largest run of rows that fits both the variant and the index budget
         int64_t vend = std::min(nv, v + ctx->chunk_variants);
@@ -466,9 +559,8 @@ int process_calls(vpca_ctx* ctx, vpca_ctx::Lane& L, const int64_t* offsets, cons
             }
             ctx->c_d2h += (nvc * bits + 7) / 8 * (int64_t)ctx->rows();
         } else {
-            int rc = launch_gram(ctx, L.plan, L.stream, L.ev_t0, L.ev_t1, L.d_x[b], nvc, P, P, d_target);
+            int rc = consume_chunk(ctx, L.plan, L.stream, L.ev_t0, L.ev_t1, *sink, L.d_x[b], v, nvc, P);
             if (rc != VPCA_OK) return rc;
-            launched = true;
         }
         CUDA_OK(ctx, cudaEventRecord(L.ev_done[b], L.stream));
         v = vend;
@@ -477,7 +569,7 @@ int process_calls(vpca_ctx* ctx, vpca_ctx::Lane& L, const int64_t* offsets, cons
     CUDA_OK(ctx, cudaMemcpyAsync(L.h_flags, L.d_flags, sizeof(int), cudaMemcpyDeviceToHost, L.stream));
     // the caller's buffers are read asynchronously: do not return before every copy has completed
     CUDA_OK(ctx, cudaStreamSynchronize(L.stream));
-    if (launched) lane_gram_time(ctx, L);
+    if (sink != nullptr && sink->launched) lane_gram_time(ctx, L);
     if (*L.h_flags & 1)
         return fail(ctx, VPCA_ERR_INDEX_OUT_OF_RANGE, "sample index outside [0, %d) (the reference throws at "
                     "VariantsPca.scala:59/:188)", ctx->rows());
@@ -487,18 +579,6 @@ int process_calls(vpca_ctx* ctx, vpca_ctx::Lane& L, const int64_t* offsets, cons
     return VPCA_OK;
 }
 
-
-template <typename T>
-static cudaError_t grow_buffer(T** p, int64_t* cap, int64_t need) {
-    if (need <= *cap && *p != nullptr) return cudaSuccess;
-    cudaFree(*p);
-    *p = nullptr;
-    *cap = 0;
-    const int64_t c = need + need / 4 + 1024;
-    cudaError_t e = cudaMalloc(p, (size_t)c * sizeof(T));
-    if (e == cudaSuccess) *cap = c;
-    return e;
-}
 
 }  // namespace
 
@@ -515,7 +595,8 @@ const char* vpca_last_error(const vpca_ctx* ctx) {
     return tls_error_copy.c_str();
 }
 
-static int create_impl(const vpca_config* cfg, int n_proj, const int32_t* sample_rows, vpca_ctx** out) {
+static int create_impl(const vpca_config* cfg, int n_proj, const int32_t* sample_rows, const vpca_model* model,
+                       vpca_ctx** out) {
     if (out == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "out is NULL");
     *out = nullptr;
     if (cfg == nullptr || cfg->struct_size != sizeof(vpca_config))
@@ -574,8 +655,35 @@ static int create_impl(const vpca_config* cfg, int n_proj, const int32_t* sample
         e = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking);
         ctx->own_stream = true;
     }
-    const size_t gram_cells = ctx->gram_cells();
-    if (e == cudaSuccess) {
+    const size_t gram_cells = model != nullptr ? 0 : ctx->gram_cells();
+    if (model != nullptr) {
+        // scoring context: the model goes to the device, and one accumulator for direct input; no Gram
+        ctx->scoring = true;
+        ctx->model_k = model->k;
+        ctx->model_nfit = model->n_fitted;
+        ctx->model_nv = model->n_variants;
+        const size_t V = (size_t)std::max<int64_t>(1, model->n_variants), k = (size_t)model->k;
+        if (e == cudaSuccess) e = cudaMalloc(&ctx->d_model_L, V * k * sizeof(double));
+        if (e == cudaSuccess) e = cudaMalloc(&ctx->d_model_n, V * sizeof(int32_t));
+        if (e == cudaSuccess) e = cudaMalloc(&ctx->d_model_terms, (3 * k + 1) * sizeof(double));
+        if (e == cudaSuccess) e = cudaMalloc(&ctx->d_direct, ctx->slot_bytes());
+        if (e == cudaSuccess && model->n_variants > 0) {
+            e = cudaMemcpy(ctx->d_model_L, model->loadings, (size_t)model->n_variants * k * sizeof(double), cudaMemcpyHostToDevice);
+            if (e == cudaSuccess)
+                e = cudaMemcpy(ctx->d_model_n, model->carriers, (size_t)model->n_variants * sizeof(int32_t), cudaMemcpyHostToDevice);
+        }
+        if (e == cudaSuccess) {
+            std::vector<double> terms(3 * k + 1);
+            for (size_t c = 0; c < k; ++c) {
+                terms[c] = model->eigenvalues[c];
+                terms[k + c] = model->col_sums[c];
+                terms[2 * k + c] = model->rowsum_dots[c];
+            }
+            terms[3 * k] = model->matrix_mean;
+            e = cudaMemcpy(ctx->d_model_terms, terms.data(), terms.size() * sizeof(double), cudaMemcpyHostToDevice);
+        }
+        if (e == cudaSuccess) e = cudaMemsetAsync(ctx->d_direct, 0, ctx->slot_bytes(), ctx->stream);
+    } else if (e == cudaSuccess) {
         if (cfg->d_gram != nullptr) {
             ctx->d_S = static_cast<int32_t*>(cfg->d_gram);
         } else {
@@ -584,7 +692,7 @@ static int create_impl(const vpca_config* cfg, int n_proj, const int32_t* sample
             if (e == cudaSuccess) e = cudaMemsetAsync(ctx->d_S + gram_cells, 0, 64 * sizeof(int32_t), ctx->stream);
         }
     }
-    if (e == cudaSuccess) e = cudaMemsetAsync(ctx->d_S, 0, gram_cells * sizeof(int32_t), ctx->stream);
+    if (e == cudaSuccess && model == nullptr) e = cudaMemsetAsync(ctx->d_S, 0, gram_cells * sizeof(int32_t), ctx->stream);
     if (e == cudaSuccess && sample_rows != nullptr) {
         e = cudaMalloc(&ctx->d_rows, (size_t)ctx->rows() * sizeof(int32_t));
         if (e == cudaSuccess)
@@ -607,7 +715,7 @@ static int create_impl(const vpca_config* cfg, int n_proj, const int32_t* sample
     return VPCA_OK;
 }
 
-int vpca_create(const vpca_config* cfg, vpca_ctx** out) { return create_impl(cfg, 0, nullptr, out); }
+int vpca_create(const vpca_config* cfg, vpca_ctx** out) { return create_impl(cfg, 0, nullptr, nullptr, out); }
 
 int vpca_create_projecting(const vpca_config* cfg, const vpca_projection* proj, vpca_ctx** out) {
     if (out != nullptr) *out = nullptr;
@@ -640,7 +748,7 @@ int vpca_create_projecting(const vpca_config* cfg, const vpca_projection* proj, 
         if (ex != nullptr && atoi(ex) != 0)
             return fail(nullptr, VPCA_ERR_UNSUPPORTED, "VPCA_EXACT_COVER=1 has no tiling of the cross block");
     }
-    return create_impl(cfg, m, identity ? nullptr : proj->sample_rows, out);
+    return create_impl(cfg, m, identity ? nullptr : proj->sample_rows, nullptr, out);
 }
 
 int vpca_destroy(vpca_ctx* ctx) {
@@ -658,6 +766,12 @@ int vpca_destroy(vpca_ctx* ctx) {
     if (ctx->own_S) cudaFree(ctx->d_S);
     cudaFree(ctx->d_rows);
     cudaFree(ctx->d_proj);
+    cudaFree(ctx->d_model_L);
+    cudaFree(ctx->d_model_n);
+    cudaFree(ctx->d_model_terms);
+    cudaFree(ctx->d_direct);
+    cudaFree(ctx->d_scratch);
+    for (auto& kv : ctx->scored) cudaFree(kv.second.d_acc);
     if (ctx->eig_ready) eig_free(ctx->eig);
     join_free(ctx->join);
     gram_plan_free(ctx->plan);
@@ -682,7 +796,15 @@ int vpca_reset(vpca_ctx* ctx) {
     for (auto& L : ctx->lanes)
         if (L.busy) return fail(ctx, VPCA_ERR_STATE, "vpca_reset while an accumulate call is in flight");
     CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
-    CUDA_OK(ctx, cudaMemsetAsync(ctx->d_S, 0, ctx->gram_cells() * sizeof(int32_t), ctx->stream));
+    if (ctx->scoring) {
+        CUDA_OK(ctx, cudaMemsetAsync(ctx->d_direct, 0, ctx->slot_bytes(), ctx->stream));
+        CUDA_OK(ctx, cudaStreamSynchronize(ctx->stream));   // no commit still reads a partial that is freed below
+        for (auto& kv : ctx->scored) cudaFree(kv.second.d_acc);
+        ctx->scored.clear();
+        ctx->direct_matched = 0;
+    } else {
+        CUDA_OK(ctx, cudaMemsetAsync(ctx->d_S, 0, ctx->gram_cells() * sizeof(int32_t), ctx->stream));
+    }
     for (auto& s : ctx->slots) s.used = false;
     ctx->finalized = false;
     ctx->pca_done = false;
@@ -709,6 +831,7 @@ int vpca_encode_calls(vpca_ctx* ctx, const int64_t* offsets, const int32_t* samp
 static int accumulate_calls_impl(vpca_ctx* ctx, int64_t partition_id, const int64_t* offsets, const void* sample_idx,
                                  int idx_bytes, int64_t nv) {
     if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    REFUSE_ON_SCORING(ctx);
     if (offsets == nullptr || nv < 0 || (nv > 0 && sample_idx == nullptr && offsets[nv] > offsets[0]))
         return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_accumulate_calls: bad argument");
     CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
@@ -724,7 +847,9 @@ static int accumulate_calls_impl(vpca_ctx* ctx, int64_t partition_id, const int6
         LaneGuard lg(ctx);
         rc = lg.rc;
         if (rc == VPCA_OK) rc = prepare_slot(ctx, *lg.lane, sc);
-        if (rc == VPCA_OK) rc = process_calls(ctx, *lg.lane, offsets, sample_idx, idx_bytes, nv, sc.target, nullptr, 0);
+        ChunkSink sink;
+        sink.gram = sc.target;
+        if (rc == VPCA_OK) rc = process_calls(ctx, *lg.lane, offsets, sample_idx, idx_bytes, nv, &sink, nullptr, 0);
     }
     return sc.end(rc);
 }
@@ -741,13 +866,50 @@ int vpca_accumulate_calls_u16(vpca_ctx* ctx, int64_t partition_id, const int64_t
     return accumulate_calls_impl(ctx, partition_id, offsets, sample_idx, 2, nv);
 }
 
-// code 0: bitmap rows; 1 / 2: PLINK .bed rows counting A1 / A2 (see encode.cu)
-static int accumulate_packed(vpca_ctx* ctx, int64_t partition_id, const uint8_t* bits, int64_t nv, int64_t stride_bytes,
-                             int code) {
-    if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+// Packed rows -> encode -> sink, on lane L.  code 0: bitmap rows; 1 / 2: PLINK .bed rows counting A1 / A2 (encode.cu).
+static int packed_chunks(vpca_ctx* ctx, vpca_ctx::Lane& L, const uint8_t* bits, int64_t nv, int64_t stride_bytes, int code,
+                         ChunkSink& sink) {
+    // bits beyond sample n-1 in the last byte of a row would be read as carriers of non-existent samples: the kernel
+    // masks them (smp >= n), nothing to validate on the host.
+    const int64_t P = ctx->panel;
+    const int64_t cap_rows = std::min<int64_t>(ctx->chunk_variants, (ctx->chunk_nnz * (int64_t)sizeof(int32_t)) / stride_bytes);
+    if (cap_rows < 32) return fail(ctx, VPCA_ERR_BAD_ARG, "stride_bytes too large for the staging buffer");
+    const int64_t whole = std::max<int64_t>(P, (cap_rows / P) * P);
+    const int64_t step = whole <= cap_rows ? whole : (cap_rows / 32) * 32;
+    int chunk = 0;
+    for (int64_t v = 0; v < nv; v += step, ++chunk) {
+        const int64_t nvc = std::min(step, nv - v);
+        const int b = chunk & 1;
+        CUDA_OK(ctx, cudaStreamWaitEvent(L.copy_stream, L.ev_done[b], 0));
+        CUDA_OK(ctx, cudaMemcpyAsync(L.d_idx[b], bits + (size_t)v * stride_bytes, (size_t)nvc * stride_bytes,
+                                     cudaMemcpyHostToDevice, L.copy_stream));
+        CUDA_OK(ctx, cudaEventRecord(L.ev_copy[b], L.copy_stream));
+        ctx->c_h2d += nvc * stride_bytes;
+        CUDA_OK(ctx, cudaStreamWaitEvent(L.stream, L.ev_copy[b], 0));
+        CUDA_OK(ctx, encode_bits(reinterpret_cast<const uint8_t*>(L.d_idx[b]), stride_bytes, nvc, ctx->rows(), ctx->elem_bits,
+                                 L.d_x[b], P, P, code, ctx->d_rows, L.stream));
+        ctx->c_launches += 1;
+        const int r = consume_chunk(ctx, L.plan, L.stream, L.ev_t0, L.ev_t1, sink, L.d_x[b], v, nvc, P);
+        if (r != VPCA_OK) return r;
+        CUDA_OK(ctx, cudaEventRecord(L.ev_done[b], L.stream));
+    }
+    CUDA_OK(ctx, cudaStreamSynchronize(L.stream));   // the caller's buffer is free to reuse on return
+    return VPCA_OK;
+}
+
+static int packed_args(vpca_ctx* ctx, const uint8_t* bits, int64_t nv, int64_t stride_bytes, int code) {
     const int64_t min_stride = code == 0 ? (ctx->rows() + 7) / 8 : (ctx->rows() + 3) / 4;
     if (nv < 0 || (nv > 0 && bits == nullptr) || stride_bytes < min_stride)
         return fail(ctx, VPCA_ERR_BAD_ARG, "packed rows: stride_bytes must be >= ceil(n_samples / %d)", code == 0 ? 8 : 4);
+    return VPCA_OK;
+}
+
+static int accumulate_packed(vpca_ctx* ctx, int64_t partition_id, const uint8_t* bits, int64_t nv, int64_t stride_bytes,
+                             int code) {
+    if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    REFUSE_ON_SCORING(ctx);
+    int rc = packed_args(ctx, bits, nv, stride_bytes, code);
+    if (rc != VPCA_OK) return rc;
     CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
     if (nv == 0) {
         std::lock_guard<std::mutex> lk(ctx->mu);
@@ -755,43 +917,16 @@ static int accumulate_packed(vpca_ctx* ctx, int64_t partition_id, const uint8_t*
         return VPCA_OK;
     }
     CallScope sc{ctx, partition_id, nv};
-    int rc = sc.begin();
+    rc = sc.begin();
     if (rc != VPCA_OK) return rc;
-    auto body = [&](vpca_ctx::Lane& L) -> int {
-        int r = prepare_slot(ctx, L, sc);
-        if (r != VPCA_OK) return r;
-        // bits beyond sample n-1 in the last byte of a row would be read as carriers of non-existent samples: the kernel
-        // masks them (smp >= n), nothing to validate on the host.
-        const int64_t P = ctx->panel;
-        const int64_t cap_rows = std::min<int64_t>(ctx->chunk_variants, (ctx->chunk_nnz * (int64_t)sizeof(int32_t)) / stride_bytes);
-        if (cap_rows < 32) return fail(ctx, VPCA_ERR_BAD_ARG, "stride_bytes too large for the staging buffer");
-        const int64_t whole = std::max<int64_t>(P, (cap_rows / P) * P);
-        const int64_t step = whole <= cap_rows ? whole : (cap_rows / 32) * 32;
-        int chunk = 0;
-        for (int64_t v = 0; v < nv; v += step, ++chunk) {
-            const int64_t nvc = std::min(step, nv - v);
-            const int b = chunk & 1;
-            CUDA_OK(ctx, cudaStreamWaitEvent(L.copy_stream, L.ev_done[b], 0));
-            CUDA_OK(ctx, cudaMemcpyAsync(L.d_idx[b], bits + (size_t)v * stride_bytes, (size_t)nvc * stride_bytes,
-                                         cudaMemcpyHostToDevice, L.copy_stream));
-            CUDA_OK(ctx, cudaEventRecord(L.ev_copy[b], L.copy_stream));
-            ctx->c_h2d += nvc * stride_bytes;
-            CUDA_OK(ctx, cudaStreamWaitEvent(L.stream, L.ev_copy[b], 0));
-            CUDA_OK(ctx, encode_bits(reinterpret_cast<const uint8_t*>(L.d_idx[b]), stride_bytes, nvc, ctx->rows(), ctx->elem_bits,
-                                     L.d_x[b], P, P, code, ctx->d_rows, L.stream));
-            ctx->c_launches += 1;
-            r = launch_gram(ctx, L.plan, L.stream, L.ev_t0, L.ev_t1, L.d_x[b], nvc, P, P, sc.target);
-            if (r != VPCA_OK) return r;
-            CUDA_OK(ctx, cudaEventRecord(L.ev_done[b], L.stream));
-        }
-        CUDA_OK(ctx, cudaStreamSynchronize(L.stream));   // the caller's buffer is free to reuse on return
-        lane_gram_time(ctx, L);
-        return VPCA_OK;
-    };
     {
         LaneGuard lg(ctx);
         rc = lg.rc;
-        if (rc == VPCA_OK) rc = body(*lg.lane);
+        if (rc == VPCA_OK) rc = prepare_slot(ctx, *lg.lane, sc);
+        ChunkSink sink;
+        sink.gram = sc.target;
+        if (rc == VPCA_OK) rc = packed_chunks(ctx, *lg.lane, bits, nv, stride_bytes, code, sink);
+        if (rc == VPCA_OK) lane_gram_time(ctx, *lg.lane);
     }
     return sc.end(rc);
 }
@@ -924,6 +1059,7 @@ int vpca_join_size(vpca_ctx* ctx, int64_t* out_rows, int64_t* out_nnz) {
 
 int vpca_accumulate_joined(vpca_ctx* ctx, int64_t partition_id) {
     if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> jl(ctx->join_mu);
     JoinWork& w = ctx->join;
     if (w.out_rows < 0) return fail(ctx, VPCA_ERR_STATE, "no joined rows: call vpca_join_rows first");
@@ -982,6 +1118,27 @@ int vpca_commit(vpca_ctx* ctx, int64_t partition_id) {
     if (s == nullptr) return VPCA_OK;   // an empty partition never staged anything
     if (s->busy) return fail(ctx, VPCA_ERR_STATE, "partition %lld still has an accumulate call in flight", (long long)partition_id);
     CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
+    if (ctx->scoring) {
+        // the partial is kept as it is, per partition id: vpca_score_project adds them in ascending id, so the result does
+        // not depend on the commit order; a partition committed again replaces its earlier partial (it counts once)
+        if (s->nv > 0) {
+            vpca_ctx::Scored& dst = ctx->scored[partition_id];
+            if (dst.d_acc == nullptr) {
+                cudaError_t e = cudaMalloc(&dst.d_acc, ctx->slot_bytes());
+                if (e != cudaSuccess) {
+                    ctx->scored.erase(partition_id);
+                    return fail(ctx, VPCA_ERR_NOMEM, "cudaMalloc of a partition score failed: %s", cudaGetErrorString(e));
+                }
+            }
+            CUDA_OK(ctx, cudaMemcpyAsync(dst.d_acc, s->d_S, ctx->slot_bytes(), cudaMemcpyDeviceToDevice, ctx->stream));
+            CUDA_OK(ctx, cudaEventRecord(s->ev_free, ctx->stream));
+            dst.matched = s->matched;
+        }
+        ctx->total_variants += s->nv;
+        ctx->inflight_variants -= s->nv;
+        s->used = false;
+        return VPCA_OK;
+    }
     // the partition's variants were reserved against the int32 bound when they were staged (CallScope::begin)
     if (s->nv > 0) {
         // every accumulate call of the partition synchronised its lane before returning: the staging Gram is complete
@@ -1016,6 +1173,7 @@ int vpca_abort(vpca_ctx* ctx, int64_t partition_id) {
 
 int vpca_accumulate_dense(vpca_ctx* ctx, const void* x, int64_t nv, int64_t ld, int on_device) {
     if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    REFUSE_ON_SCORING(ctx);
     if (x == nullptr || nv < 0 || ld < nv) return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_accumulate_dense: bad argument");
     const int bits = ctx->elem_bits;
     if (bits == 4 && (ld % 128) != 0)
@@ -1083,6 +1241,7 @@ int vpca_accumulate_dense(vpca_ctx* ctx, const void* x, int64_t nv, int64_t ld, 
 
 int vpca_accumulate_panels(vpca_ctx* ctx, const void* d_x, int64_t nv, int64_t panel_variants) {
     if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (d_x == nullptr || nv < 0 || panel_variants < 128 || (panel_variants % 128) != 0)
         return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_accumulate_panels: panel_variants must be a positive multiple of 128");
@@ -1096,7 +1255,9 @@ int vpca_accumulate_panels(vpca_ctx* ctx, const void* d_x, int64_t nv, int64_t p
     if (nv == 0) return VPCA_OK;
     int rc = check_overflow(ctx, nv);
     if (rc != VPCA_OK) return rc;
-    rc = launch_gram(ctx, ctx->plan, ctx->stream, ctx->ev_t0, ctx->ev_t1, d_x, nv, panel_variants, panel_variants, ctx->d_S);
+    ChunkSink sink;
+    sink.gram = ctx->d_S;
+    rc = consume_chunk(ctx, ctx->plan, ctx->stream, ctx->ev_t0, ctx->ev_t1, sink, d_x, 0, nv, panel_variants);
     if (rc != VPCA_OK) return rc;
     ctx->gram_timed = true;
     ctx->st.gram_cta_group = ctx->plan.cta_group;
@@ -1122,12 +1283,14 @@ int vpca_synth_panels_device(vpca_ctx* ctx, uint64_t seed, int64_t v0, int64_t n
 
 int vpca_gram_device_ptr(vpca_ctx* ctx, void** d_gram) {
     if (ctx == nullptr || d_gram == nullptr) return fail(ctx, VPCA_ERR_BAD_ARG, "NULL argument");
+    REFUSE_ON_SCORING(ctx);
     *d_gram = ctx->d_S;
     return VPCA_OK;
 }
 
 int vpca_finalize_gram(vpca_ctx* ctx) {
     if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (ctx->finalized) return VPCA_OK;
     for (auto& s : ctx->slots)
@@ -1156,6 +1319,7 @@ static int copy_gram_out(vpca_ctx* ctx, int32_t* out, size_t cells) {
 
 int vpca_get_gram(vpca_ctx* ctx, int32_t* out) {
     if (ctx == nullptr || out == nullptr) return fail(ctx, VPCA_ERR_BAD_ARG, "NULL argument");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (!ctx->finalized) return fail(ctx, VPCA_ERR_STATE, "call vpca_finalize_gram first");
     if (ctx->band_rows != ctx->n) return fail(ctx, VPCA_ERR_STATE, "this context stores a row band: use vpca_get_gram_band");
@@ -1164,6 +1328,7 @@ int vpca_get_gram(vpca_ctx* ctx, int32_t* out) {
 
 int vpca_get_gram_band(vpca_ctx* ctx, int32_t row0, int32_t rows, int32_t* out) {
     if (ctx == nullptr || out == nullptr) return fail(ctx, VPCA_ERR_BAD_ARG, "NULL argument");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (rows <= 0 || row0 < ctx->band_row0 || row0 + rows > ctx->band_row0 + ctx->band_rows)
         return fail(ctx, VPCA_ERR_BAD_ARG, "rows [%d, %d) are outside the band [%d, %d) this context stores", row0, row0 + rows,
@@ -1179,6 +1344,7 @@ int vpca_get_gram_band(vpca_ctx* ctx, int32_t row0, int32_t rows, int32_t* out) 
 
 int vpca_get_partial_gram(vpca_ctx* ctx, int32_t* out, int64_t* variants_in_gram) {
     if (ctx == nullptr || out == nullptr) return fail(ctx, VPCA_ERR_BAD_ARG, "NULL argument");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (ctx->finalized) return fail(ctx, VPCA_ERR_STATE, "Gram already finalized: use vpca_get_gram");
     if (ctx->band_rows != ctx->n) return fail(ctx, VPCA_ERR_STATE, "this context stores a row band: use vpca_get_gram_band");
@@ -1188,6 +1354,7 @@ int vpca_get_partial_gram(vpca_ctx* ctx, int32_t* out, int64_t* variants_in_gram
 
 int vpca_load_partial_gram(vpca_ctx* ctx, const int32_t* gram, int64_t variants_in_gram) {
     if (ctx == nullptr || gram == nullptr || variants_in_gram < 0) return fail(ctx, VPCA_ERR_BAD_ARG, "bad argument");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (ctx->finalized) return fail(ctx, VPCA_ERR_STATE, "Gram already finalized; call vpca_reset first");
     if (ctx->band_rows != ctx->n) return fail(ctx, VPCA_ERR_STATE, "this context stores a row band");
@@ -1206,6 +1373,7 @@ int vpca_load_partial_gram(vpca_ctx* ctx, const int32_t* gram, int64_t variants_
 
 int vpca_set_gram(vpca_ctx* ctx, const int32_t* gram) {
     if (ctx == nullptr || gram == nullptr) return fail(ctx, VPCA_ERR_BAD_ARG, "NULL argument");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (ctx->band_rows != ctx->n) return fail(ctx, VPCA_ERR_STATE, "this context stores a row band");
     if (ctx->n_proj > 0)
@@ -1245,6 +1413,7 @@ static int run_center(vpca_ctx* ctx, bool materialise) {
 
 int vpca_compute_pca(vpca_ctx* ctx, int32_t k, double* vecs, double* evals, int32_t* non_zero_rows) {
     if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (vecs == nullptr || k < 1 || k > ctx->n || k > std::max(ctx->num_pc, 16))
         return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_compute_pca: k=%d out of range", k);
@@ -1283,6 +1452,7 @@ int vpca_compute_pca(vpca_ctx* ctx, int32_t k, double* vecs, double* evals, int3
 
 int vpca_get_cross_gram(vpca_ctx* ctx, int32_t* out) {
     if (ctx == nullptr || out == nullptr) return fail(ctx, VPCA_ERR_BAD_ARG, "NULL argument");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (!ctx->finalized) return fail(ctx, VPCA_ERR_STATE, "call vpca_finalize_gram first");
     if (ctx->n_proj == 0) return VPCA_OK;
@@ -1297,6 +1467,7 @@ int vpca_get_cross_gram(vpca_ctx* ctx, int32_t* out) {
 
 int vpca_project_pca(vpca_ctx* ctx, int32_t k, double* out) {
     if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (ctx->proj_k == 0) return fail(ctx, VPCA_ERR_STATE, "call vpca_compute_pca first");
     if (k < 1 || k > ctx->proj_k)
@@ -1325,6 +1496,272 @@ int vpca_project_pca(vpca_ctx* ctx, int32_t k, double* out) {
     return VPCA_OK;
 }
 
+// ---- saved model: loadings of a fitted context, scoring of a study context (model.cu) -------------------------------
+static int loadings_args(vpca_ctx* ctx, int32_t k, int64_t nv, const double* loadings, const int32_t* carriers) {
+    if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    REFUSE_ON_SCORING(ctx);
+    if (nv < 0 || (nv > 0 && (loadings == nullptr || carriers == nullptr)))
+        return fail(ctx, VPCA_ERR_BAD_ARG, "loadings: nv must be >= 0 and the outputs non-NULL");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (ctx->proj_k == 0) return fail(ctx, VPCA_ERR_STATE, "call vpca_compute_pca first");
+    if (k < 1 || k > ctx->proj_k)
+        return fail(ctx, VPCA_ERR_BAD_ARG, "loadings: k=%d outside [1, %d] (the k of the last vpca_compute_pca)", k, ctx->proj_k);
+    return VPCA_OK;
+}
+
+static size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
+
+// Loadings sink of a lane: device output for one chunk in the lane's scratch.
+static int lane_loadings_sink(vpca_ctx* ctx, vpca_ctx::Lane& L, int32_t k, double* loadings, int32_t* carriers, ChunkSink& sink) {
+    const int64_t cv = ctx->chunk_variants;
+    const size_t lb = align256((size_t)cv * k * sizeof(double));
+    CUDA_OK(ctx, grow_buffer(&L.d_scratch, &L.cap_scratch, (int64_t)(lb + (size_t)cv * sizeof(int32_t))));
+    sink.kind = ChunkSink::LOADINGS;
+    sink.k = k;
+    sink.d_L = reinterpret_cast<double*>(L.d_scratch);
+    sink.d_cnt = reinterpret_cast<int32_t*>(L.d_scratch + lb);
+    sink.h_L = loadings;
+    sink.h_cnt = carriers;
+    return VPCA_OK;
+}
+
+int vpca_pca_loadings_calls(vpca_ctx* ctx, int32_t k, const int64_t* offsets, const int32_t* sample_idx, int64_t nv,
+                            double* loadings, int32_t* carriers) {
+    int rc = loadings_args(ctx, k, nv, loadings, carriers);
+    if (rc != VPCA_OK) return rc;
+    if (offsets == nullptr || (nv > 0 && sample_idx == nullptr && offsets[nv] > offsets[0]))
+        return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_pca_loadings_calls: bad argument");
+    CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
+    if (nv == 0) return VPCA_OK;
+    LaneGuard lg(ctx);
+    if (lg.rc != VPCA_OK) return lg.rc;
+    ChunkSink sink;
+    rc = lane_loadings_sink(ctx, *lg.lane, k, loadings, carriers, sink);
+    if (rc != VPCA_OK) return rc;
+    return process_calls(ctx, *lg.lane, offsets, sample_idx, 4, nv, &sink, nullptr, 0);
+}
+
+int vpca_pca_loadings_bed(vpca_ctx* ctx, int32_t k, const uint8_t* rows, int64_t nv, int64_t stride_bytes,
+                          int32_t counted_allele, double* loadings, int32_t* carriers) {
+    int rc = loadings_args(ctx, k, nv, loadings, carriers);
+    if (rc != VPCA_OK) return rc;
+    if (counted_allele != 1 && counted_allele != 2)
+        return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_pca_loadings_bed: counted_allele must be 1 (A1) or 2 (A2)");
+    rc = packed_args(ctx, rows, nv, stride_bytes, counted_allele);
+    if (rc != VPCA_OK) return rc;
+    CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
+    if (nv == 0) return VPCA_OK;
+    LaneGuard lg(ctx);
+    if (lg.rc != VPCA_OK) return lg.rc;
+    ChunkSink sink;
+    rc = lane_loadings_sink(ctx, *lg.lane, k, loadings, carriers, sink);
+    if (rc != VPCA_OK) return rc;
+    return packed_chunks(ctx, *lg.lane, rows, nv, stride_bytes, counted_allele, sink);
+}
+
+static int panels_args(vpca_ctx* ctx, const void* d_x, int64_t nv, int64_t panel_variants) {
+    if (d_x == nullptr || nv < 0 || panel_variants < 128 || (panel_variants % 128) != 0)
+        return fail(ctx, VPCA_ERR_BAD_ARG, "panels: panel_variants must be a positive multiple of 128");
+    if ((reinterpret_cast<uintptr_t>(d_x) & 31) != 0) return fail(ctx, VPCA_ERR_BAD_ARG, "panels must be 32-byte aligned");
+    return VPCA_OK;
+}
+
+int vpca_pca_loadings_panels(vpca_ctx* ctx, int32_t k, const void* d_x, int64_t nv, int64_t panel_variants, double* loadings,
+                             int32_t* carriers) {
+    int rc = loadings_args(ctx, k, nv, loadings, carriers);
+    if (rc != VPCA_OK) return rc;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    rc = panels_args(ctx, d_x, nv, panel_variants);
+    if (rc != VPCA_OK) return rc;
+    CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
+    if (nv == 0) return VPCA_OK;
+    const size_t lb = align256((size_t)nv * k * sizeof(double));
+    CUDA_OK(ctx, grow_buffer(&ctx->d_scratch, &ctx->cap_scratch, (int64_t)(lb + (size_t)nv * sizeof(int32_t))));
+    ChunkSink sink;
+    sink.kind = ChunkSink::LOADINGS;
+    sink.k = k;
+    sink.d_L = reinterpret_cast<double*>(ctx->d_scratch);
+    sink.d_cnt = reinterpret_cast<int32_t*>(ctx->d_scratch + lb);
+    sink.h_L = loadings;
+    sink.h_cnt = carriers;
+    rc = consume_chunk(ctx, ctx->plan, ctx->stream, ctx->ev_t0, ctx->ev_t1, sink, d_x, 0, nv, panel_variants);
+    if (rc != VPCA_OK) return rc;
+    CUDA_OK(ctx, cudaStreamSynchronize(ctx->stream));
+    return VPCA_OK;
+}
+
+int vpca_pca_model_terms(vpca_ctx* ctx, int32_t k, double* eigenvalues, double* col_sums, double* rowsum_dots,
+                         double* matrix_mean) {
+    int rc = loadings_args(ctx, k, 0, nullptr, nullptr);
+    if (rc != VPCA_OK) return rc;
+    if (eigenvalues == nullptr || col_sums == nullptr || rowsum_dots == nullptr || matrix_mean == nullptr)
+        return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_pca_model_terms: NULL argument");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
+    CUDA_OK(ctx, grow_buffer(&ctx->d_scratch, &ctx->cap_scratch, (int64_t)(2 * k * sizeof(double))));
+    double* d_a = reinterpret_cast<double*>(ctx->d_scratch);
+    CUDA_OK(ctx, model_terms(ctx->eig.d_evecs, ctx->eig.d_rowsum, ctx->n, k, d_a, d_a + k, ctx->stream));
+    ctx->c_launches += 1;
+    CUDA_OK(ctx, cudaMemcpyAsync(col_sums, d_a, k * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_OK(ctx, cudaMemcpyAsync(rowsum_dots, d_a + k, k * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_OK(ctx, cudaMemcpyAsync(eigenvalues, ctx->eig.d_evals, k * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_OK(ctx, cudaMemcpyAsync(matrix_mean, ctx->eig.d_mm, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_OK(ctx, cudaStreamSynchronize(ctx->stream));
+    ctx->c_d2h += (3 * k + 1) * 8;
+    return VPCA_OK;
+}
+
+int vpca_create_scoring(const vpca_config* cfg, const vpca_model* model, vpca_ctx** out) {
+    if (out != nullptr) *out = nullptr;
+    if (model == nullptr || model->struct_size != sizeof(vpca_model))
+        return fail(nullptr, VPCA_ERR_BAD_ARG, "model is NULL or struct_size != sizeof(vpca_model) (%zu)", sizeof(vpca_model));
+    if (model->n_fitted < 2 || model->k < 1 || model->n_variants < 0 || model->n_variants > 0x7fffffffll)
+        return fail(nullptr, VPCA_ERR_BAD_ARG, "model: need n_fitted >= 2, k >= 1 and 0 <= n_variants < 2^31");
+    if ((model->n_variants > 0 && (model->loadings == nullptr || model->carriers == nullptr)) || model->eigenvalues == nullptr ||
+        model->col_sums == nullptr || model->rowsum_dots == nullptr)
+        return fail(nullptr, VPCA_ERR_BAD_ARG, "model: NULL array");
+    if (cfg != nullptr && cfg->struct_size == sizeof(vpca_config) && (cfg->d_gram != nullptr || cfg->gram_band_rows > 0))
+        return fail(nullptr, VPCA_ERR_BAD_ARG, "a scoring context has no Gram: d_gram and gram_band_rows must be unset");
+    return create_impl(cfg, 0, nullptr, model, out);
+}
+
+// Validates the model rows of a scoring call and counts the variants that have one.
+static int score_args(vpca_ctx* ctx, int64_t nv, const int32_t* model_rows, int64_t* matched) {
+    if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    if (!ctx->scoring) return fail(ctx, VPCA_ERR_UNSUPPORTED, "scoring needs a context made by vpca_create_scoring");
+    if (nv < 0 || (nv > 0 && model_rows == nullptr)) return fail(ctx, VPCA_ERR_BAD_ARG, "scoring: bad argument");
+    int64_t cnt = 0;
+    for (int64_t q = 0; q < nv; ++q) {
+        const int32_t r = model_rows[q];
+        if (r < -1 || r >= ctx->model_nv)
+            return fail(ctx, VPCA_ERR_INDEX_OUT_OF_RANGE, "model row %d of variant %lld is outside [-1, %lld)", r, (long long)q,
+                        (long long)ctx->model_nv);
+        cnt += r >= 0;
+    }
+    *matched = cnt;
+    return VPCA_OK;
+}
+
+// Scoring sink: the model rows of the call are copied to the device once, next to the scratch of model_score.
+static int score_sink(vpca_ctx* ctx, char** buf, int64_t* cap, cudaStream_t stream, const int32_t* model_rows, int64_t nv,
+                      double* acc, ChunkSink& sink) {
+    const size_t rb = align256((size_t)nv * sizeof(int32_t));
+    CUDA_OK(ctx, grow_buffer(buf, cap, (int64_t)(rb + model_score_scratch(ctx->n, ctx->model_k))));
+    CUDA_OK(ctx, cudaMemcpyAsync(*buf, model_rows, (size_t)nv * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
+    ctx->c_h2d += nv * 4;
+    sink.kind = ChunkSink::SCORE;
+    sink.k = ctx->model_k;
+    sink.d_mrows = reinterpret_cast<const int32_t*>(*buf);
+    sink.d_part = reinterpret_cast<double*>(*buf + rb);
+    sink.d_acc = acc;
+    return VPCA_OK;
+}
+
+// Partition bookkeeping of the host-input scoring routes (commit / abort as for the Gram); `body` runs the chunk loop.
+extern "C++" template <typename Body>
+int score_on_lane(vpca_ctx* ctx, int64_t partition_id, int64_t nv, int64_t matched, const int32_t* model_rows, Body&& body) {
+    std::unique_lock<std::mutex> direct;   // direct input adds into one accumulator, one call at a time, in call order
+    if (partition_id < 0) direct = std::unique_lock<std::mutex>(ctx->direct_mu);
+    CallScope sc{ctx, partition_id, nv};
+    sc.matched = matched;
+    int rc = sc.begin();
+    if (rc != VPCA_OK) return rc;
+    {
+        LaneGuard lg(ctx);
+        rc = lg.rc;
+        if (rc == VPCA_OK) rc = prepare_slot(ctx, *lg.lane, sc);
+        ChunkSink sink;
+        if (rc == VPCA_OK)
+            rc = score_sink(ctx, &lg.lane->d_scratch, &lg.lane->cap_scratch, lg.lane->stream, model_rows, nv,
+                            reinterpret_cast<double*>(sc.target), sink);
+        if (rc == VPCA_OK) rc = body(*lg.lane, sink);
+    }
+    return sc.end(rc);
+}
+
+int vpca_score_calls(vpca_ctx* ctx, int64_t partition_id, const int64_t* offsets, const int32_t* sample_idx, int64_t nv,
+                     const int32_t* model_rows) {
+    int64_t matched = 0;
+    int rc = score_args(ctx, nv, model_rows, &matched);
+    if (rc != VPCA_OK) return rc;
+    if (offsets == nullptr || (nv > 0 && sample_idx == nullptr && offsets[nv] > offsets[0]))
+        return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_score_calls: bad argument");
+    CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
+    if (nv == 0) return VPCA_OK;
+    return score_on_lane(ctx, partition_id, nv, matched, model_rows, [&](vpca_ctx::Lane& L, ChunkSink& sink) {
+        return process_calls(ctx, L, offsets, sample_idx, 4, nv, &sink, nullptr, 0);
+    });
+}
+
+int vpca_score_bed(vpca_ctx* ctx, int64_t partition_id, const uint8_t* rows, int64_t nv, int64_t stride_bytes,
+                   int32_t counted_allele, const int32_t* model_rows) {
+    int64_t matched = 0;
+    int rc = score_args(ctx, nv, model_rows, &matched);
+    if (rc != VPCA_OK) return rc;
+    if (counted_allele != 1 && counted_allele != 2)
+        return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_score_bed: counted_allele must be 1 (A1) or 2 (A2)");
+    rc = packed_args(ctx, rows, nv, stride_bytes, counted_allele);
+    if (rc != VPCA_OK) return rc;
+    CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
+    if (nv == 0) return VPCA_OK;
+    return score_on_lane(ctx, partition_id, nv, matched, model_rows, [&](vpca_ctx::Lane& L, ChunkSink& sink) {
+        return packed_chunks(ctx, L, rows, nv, stride_bytes, counted_allele, sink);
+    });
+}
+
+int vpca_score_panels(vpca_ctx* ctx, const void* d_x, int64_t nv, int64_t panel_variants, const int32_t* model_rows) {
+    int64_t matched = 0;
+    int rc = score_args(ctx, nv, model_rows, &matched);
+    if (rc != VPCA_OK) return rc;
+    std::lock_guard<std::mutex> dl(ctx->direct_mu);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    rc = panels_args(ctx, d_x, nv, panel_variants);
+    if (rc != VPCA_OK) return rc;
+    CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
+    if (nv == 0) return VPCA_OK;
+    ChunkSink sink;
+    rc = score_sink(ctx, &ctx->d_scratch, &ctx->cap_scratch, ctx->stream, model_rows, nv, ctx->d_direct, sink);
+    if (rc == VPCA_OK) rc = consume_chunk(ctx, ctx->plan, ctx->stream, ctx->ev_t0, ctx->ev_t1, sink, d_x, 0, nv, panel_variants);
+    if (rc != VPCA_OK) return rc;
+    ctx->total_variants += nv;
+    ctx->st.variants_accumulated += nv;
+    ctx->direct_matched += matched;
+    return VPCA_OK;
+}
+
+int vpca_score_project(vpca_ctx* ctx, int32_t k, double* out, int64_t* matched_variants) {
+    if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    if (!ctx->scoring) return fail(ctx, VPCA_ERR_UNSUPPORTED, "vpca_score_project needs a context made by vpca_create_scoring");
+    std::lock_guard<std::mutex> dl(ctx->direct_mu);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (k < 1 || k > ctx->model_k) return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_score_project: k=%d outside [1, %d]", k, ctx->model_k);
+    if (out == nullptr) return fail(ctx, VPCA_ERR_BAD_ARG, "out is NULL");
+    for (auto& s : ctx->slots)
+        if (s.used) return fail(ctx, VPCA_ERR_STATE, "partition %lld is neither committed nor aborted", (long long)s.pid);
+    for (auto& L : ctx->lanes)
+        if (L.busy) return fail(ctx, VPCA_ERR_STATE, "vpca_score_project while a scoring call is in flight");
+    CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));
+    const int m = ctx->n, K = ctx->model_k;
+    const size_t ab = align256(ctx->slot_bytes());
+    CUDA_OK(ctx, grow_buffer(&ctx->d_scratch, &ctx->cap_scratch, (int64_t)(ab + (size_t)m * k * sizeof(double))));
+    double* d_sum = reinterpret_cast<double*>(ctx->d_scratch);
+    double* d_y = reinterpret_cast<double*>(ctx->d_scratch + ab);
+    // direct input first, then the committed partitions in ascending id
+    CUDA_OK(ctx, cudaMemcpyAsync(d_sum, ctx->d_direct, ctx->slot_bytes(), cudaMemcpyDeviceToDevice, ctx->stream));
+    int64_t cnt = ctx->direct_matched;
+    for (auto& kv : ctx->scored) {
+        CUDA_OK(ctx, model_add(d_sum, kv.second.d_acc, m, K, ctx->stream));
+        cnt += kv.second.matched;
+    }
+    CUDA_OK(ctx, model_finish(d_sum, m, K, k, ctx->model_nfit, ctx->d_model_terms, d_y, ctx->stream));
+    ctx->c_launches += (int64_t)ctx->scored.size() + 1;
+    CUDA_OK(ctx, cudaMemcpyAsync(out, d_y, (size_t)m * k * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_OK(ctx, cudaStreamSynchronize(ctx->stream));
+    ctx->c_d2h += (int64_t)m * k * 8;
+    if (matched_variants != nullptr) *matched_variants = cnt;
+    return VPCA_OK;
+}
+
 int vpca_debug_projection_tiles(int32_t n_fit, int32_t n_total, int32_t cta_group, int32_t mxf4, int32_t* out,
                                 int32_t max_tiles) {
     if (n_fit < 1 || n_total < n_fit || max_tiles < 0 || (out == nullptr && max_tiles > 0))
@@ -1334,6 +1771,7 @@ int vpca_debug_projection_tiles(int32_t n_fit, int32_t n_total, int32_t cta_grou
 
 int vpca_get_centered(vpca_ctx* ctx, double* out) {
     if (ctx == nullptr || out == nullptr) return fail(ctx, VPCA_ERR_BAD_ARG, "NULL argument");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (!ctx->finalized) return fail(ctx, VPCA_ERR_STATE, "call vpca_finalize_gram first");
     if (ctx->band_rows != ctx->n) return fail(ctx, VPCA_ERR_STATE, "this context stores a row band of the Gram");
@@ -1350,6 +1788,7 @@ int vpca_get_centered(vpca_ctx* ctx, double* out) {
 
 int vpca_get_tridiagonal(vpca_ctx* ctx, double* diag, double* offdiag) {
     if (ctx == nullptr || diag == nullptr || offdiag == nullptr) return fail(ctx, VPCA_ERR_BAD_ARG, "NULL argument");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (!ctx->pca_done) return fail(ctx, VPCA_ERR_STATE, "call vpca_compute_pca first");
     if (ctx->eig.last_method == 2)
@@ -1399,6 +1838,7 @@ int vpca_get_stats(vpca_ctx* ctx, vpca_stats* out) {
 
 int vpca_gram_export_ipc(vpca_ctx* ctx, void* handle64) {
     if (ctx == nullptr || handle64 == nullptr) return fail(ctx, VPCA_ERR_BAD_ARG, "NULL argument");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (ctx->n_proj > 0) return fail(ctx, VPCA_ERR_UNSUPPORTED, "projecting contexts reduce through vpca_gram_device_ptr");
     if (!ctx->own_S) return fail(ctx, VPCA_ERR_STATE, "the peer-reduce mode needs a library-owned Gram (vpca_config.d_gram == NULL)");
@@ -1414,6 +1854,7 @@ int vpca_gram_export_ipc(vpca_ctx* ctx, void* handle64) {
 int vpca_gram_set_peers(vpca_ctx* ctx, const void* handles, int32_t world, int32_t rank) {
     if (ctx == nullptr || handles == nullptr || world < 1 || world > 16 || rank < 0 || rank >= world)
         return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_gram_set_peers: bad argument (world <= 16)");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (ctx->n_proj > 0) return fail(ctx, VPCA_ERR_UNSUPPORTED, "projecting contexts reduce through vpca_gram_device_ptr");
     if (!ctx->own_S) return fail(ctx, VPCA_ERR_STATE, "the peer-reduce mode needs a library-owned Gram");
@@ -1455,6 +1896,7 @@ int vpca_gram_set_peers_local(vpca_ctx* const* ctxs, int32_t world) {
     if (ctxs == nullptr || world < 1 || world > 16) return fail(nullptr, VPCA_ERR_BAD_ARG, "vpca_gram_set_peers_local: world must be in [1, 16]");
     for (int r = 0; r < world; ++r) {
         if (ctxs[r] == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctxs[%d] is NULL", r);
+        REFUSE_ON_SCORING(ctxs[r]);
         if (ctxs[r]->n_proj > 0)
             return fail(ctxs[r], VPCA_ERR_UNSUPPORTED, "projecting contexts reduce through vpca_gram_device_ptr");
         if (!ctxs[r]->own_S) return fail(ctxs[r], VPCA_ERR_STATE, "the peer-reduce mode needs a library-owned Gram");
@@ -1511,6 +1953,7 @@ int vpca_gram_set_peers_local(vpca_ctx* const* ctxs, int32_t world) {
 
 int vpca_gram_set_peer_mode(vpca_ctx* ctx, int32_t mode) {
     if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (mode != VPCA_PEER_REPLICATE && mode != VPCA_PEER_OWNER_ROWS)
         return fail(ctx, VPCA_ERR_BAD_ARG, "vpca_gram_set_peer_mode: unknown mode %d", mode);
@@ -1556,6 +1999,7 @@ int vpca_owner_row_bands(int32_t n_samples, int32_t world, int32_t* row_end) {
 
 int vpca_gram_gather(vpca_ctx* ctx) {
     if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (ctx->finalized) return fail(ctx, VPCA_ERR_STATE, "Gram already finalized");
     if (ctx->plan.num_peers < 2) return VPCA_OK;
@@ -1572,6 +2016,7 @@ int vpca_gram_gather(vpca_ctx* ctx) {
 
 int vpca_peer_barrier(vpca_ctx* ctx) {
     if (ctx == nullptr) return fail(nullptr, VPCA_ERR_BAD_ARG, "ctx is NULL");
+    REFUSE_ON_SCORING(ctx);
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (ctx->plan.num_peers < 2) return VPCA_OK;
     CUDA_OK(ctx, cudaSetDevice(ctx->cfg.device));

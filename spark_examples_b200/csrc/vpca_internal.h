@@ -188,6 +188,25 @@ int proj_chunks(int n);
 cudaError_t eig_project(const EigWork& w, const int32_t* d_X, int m, int k, double* d_rowmean, double* d_part, double* d_y,
                         cudaStream_t stream);
 
+// ---- saved model: loadings and scoring (model.cu) --------------------------------------------------------------
+// Every kernel reads an encoded chunk in panel layout: ceil(nv / panel) panels of `rows` x panel cells, zero after nv.
+// Loadings of the nv variants of a chunk from its rows [0, n_fit) and the first k columns of U (n_fit x k, column-major,
+// EigWork::d_evecs): d_L (nv x k row-major) and d_carriers (nv).  Fixed order over f: bit-identical for any chunking.
+cudaError_t model_loadings(const void* d_x, int elem_bits, int64_t nv, int64_t panel, int rows, int n_fit, const double* d_u,
+                           int k, double* d_L, int32_t* d_carriers, cudaStream_t stream);
+// Scoring of a chunk of m study samples (rows = m): d_acc (m x k doubles, then m int64) += (T, r) of the chunk, where
+// variant v uses model row d_mrows[v] of d_L (V x k) / d_n (-1: skipped).  d_scratch: model_score_scratch(m, k) bytes.
+size_t model_score_scratch(int m, int k);
+cudaError_t model_score(const void* d_x, int elem_bits, int64_t nv, int64_t panel, int m, const int32_t* d_mrows,
+                        const double* d_L, const int32_t* d_n, int k, double* d_scratch, double* d_acc, cudaStream_t stream);
+// a_c = sum_f u_fc and b_c = sum_f (rs_f / n) u_fc for c < k, fixed order.
+cudaError_t model_terms(const double* d_u, const double* d_rowsum, int n, int k, double* d_a, double* d_b, cudaStream_t stream);
+// d_dst += d_src, both accumulators of m samples and k columns (doubles, then int64).
+cudaError_t model_add(double* d_dst, const double* d_src, int m, int k, cudaStream_t stream);
+// d_y (m x kout, column-major) from an accumulator of k columns and d_terms = {lambda[k], a[k], b[k], matrix mean}.
+cudaError_t model_finish(const double* d_acc, int m, int k, int kout, int n_fit, const double* d_terms, double* d_y,
+                         cudaStream_t stream);
+
 // ---- synthetic generator (synth.cu) ----------------------------------------------------------------
 cudaError_t synth_dense(uint64_t seed, int n, int64_t v0, int64_t nv, int mode, int elem_bits, void* d_x,
                         int64_t ld, int64_t panel, cudaStream_t stream);

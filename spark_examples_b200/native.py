@@ -51,6 +51,8 @@ EXPORTED_SYMBOLS = (
     "vpca_pool_commit", "vpca_pool_abort", "vpca_pool_reduce_and_finalize", "vpca_pool_get_gram", "vpca_pool_compute_pca",
     "vpca_pool_get_stats", "vpca_debug_tiles", "vpca_debug_plan",
     "vpca_create_projecting", "vpca_get_cross_gram", "vpca_project_pca", "vpca_debug_projection_tiles",
+    "vpca_pca_loadings_calls", "vpca_pca_loadings_bed", "vpca_pca_loadings_panels", "vpca_pca_model_terms",
+    "vpca_create_scoring", "vpca_score_calls", "vpca_score_bed", "vpca_score_panels", "vpca_score_project",
 )
 
 
@@ -90,6 +92,21 @@ class VpcaProjection(ctypes.Structure):
         ("struct_size", ctypes.c_uint32),
         ("n_projected", ctypes.c_int32),
         ("sample_rows", ctypes.POINTER(ctypes.c_int32)),
+    ]
+
+
+class VpcaModel(ctypes.Structure):
+    _fields_ = [
+        ("struct_size", ctypes.c_uint32),
+        ("n_fitted", ctypes.c_int32),
+        ("k", ctypes.c_int32),
+        ("n_variants", ctypes.c_int64),
+        ("loadings", ctypes.c_void_p),
+        ("carriers", ctypes.c_void_p),
+        ("eigenvalues", ctypes.c_void_p),
+        ("col_sums", ctypes.c_void_p),
+        ("rowsum_dots", ctypes.c_void_p),
+        ("matrix_mean", ctypes.c_double),
     ]
 
 
@@ -265,6 +282,24 @@ def load_library() -> ctypes.CDLL:
     L.vpca_project_pca.argtypes = [vp, i32, vp]
     L.vpca_debug_projection_tiles.restype = ctypes.c_int
     L.vpca_debug_projection_tiles.argtypes = [i32, i32, i32, i32, vp, i32]
+    L.vpca_pca_loadings_calls.restype = ctypes.c_int
+    L.vpca_pca_loadings_calls.argtypes = [vp, i32, vp, vp, i64, vp, vp]
+    L.vpca_pca_loadings_bed.restype = ctypes.c_int
+    L.vpca_pca_loadings_bed.argtypes = [vp, i32, vp, i64, i64, i32, vp, vp]
+    L.vpca_pca_loadings_panels.restype = ctypes.c_int
+    L.vpca_pca_loadings_panels.argtypes = [vp, i32, vp, i64, i64, vp, vp]
+    L.vpca_pca_model_terms.restype = ctypes.c_int
+    L.vpca_pca_model_terms.argtypes = [vp, i32, vp, vp, vp, vp]
+    L.vpca_create_scoring.restype = ctypes.c_int
+    L.vpca_create_scoring.argtypes = [ctypes.POINTER(VpcaConfig), ctypes.POINTER(VpcaModel), ctypes.POINTER(vp)]
+    L.vpca_score_calls.restype = ctypes.c_int
+    L.vpca_score_calls.argtypes = [vp, i64, vp, vp, i64, vp]
+    L.vpca_score_bed.restype = ctypes.c_int
+    L.vpca_score_bed.argtypes = [vp, i64, vp, i64, i64, i32, vp]
+    L.vpca_score_panels.restype = ctypes.c_int
+    L.vpca_score_panels.argtypes = [vp, vp, i64, i64, vp]
+    L.vpca_score_project.restype = ctypes.c_int
+    L.vpca_score_project.argtypes = [vp, i32, vp, ctypes.POINTER(i64)]
     _lib = L
     return L
 
@@ -279,10 +314,13 @@ class NativePca:
     def __init__(self, n_samples: int, device: int = 0, dtype: int = DTYPE_I8, num_pc: int = 2,
                  max_multiplicity: int = 2, partitions_in_flight: int = 4, chunk_variants: int = 0,
                  chunk_nnz: int = 0, stream: int = 0, d_gram: int = 0, staging_lanes: int = 0,
-                 gram_band: Optional[Tuple[int, int]] = None, n_projected: int = 0, sample_rows=None):
+                 gram_band: Optional[Tuple[int, int]] = None, n_projected: int = 0, sample_rows=None, model=None):
         """n_projected > 0 (or a sample_rows map): a projecting context (vpca_create_projecting) -- n_samples fitted
         samples plus n_projected ones placed on the fitted PCs by projectPca.  sample_rows: input sample position ->
-        row of the context (fitted rows first), None = the last n_projected inputs are the projected ones."""
+        row of the context (fitted rows first), None = the last n_projected inputs are the projected ones.
+        model: a scoring context (vpca_create_scoring) for n_samples study samples -- an object with the fields of
+        vpca_model (n_fitted, loadings (V, k), carriers (V,), eigenvalues, col_sums, rowsum_dots (k,), matrix_mean),
+        such as model.PcaModel; it has no Gram, only the score* methods."""
         self._lib = load_library()
         self.n = int(n_samples)
         self.n_projected = int(n_projected)
@@ -296,7 +334,20 @@ class NativePca:
                          partitions_in_flight, staging_lanes, chunk_variants, chunk_nnz, stream or None, d_gram or None,
                          row0, rows)
         handle = ctypes.c_void_p()
-        if self.n_projected > 0 or sample_rows is not None:
+        self.model_k = 0
+        if model is not None:
+            L = np.ascontiguousarray(model.loadings, dtype=np.float64)
+            n_var, k = L.shape
+            cnt = np.ascontiguousarray(model.carriers, dtype=np.int32)
+            terms = [np.ascontiguousarray(getattr(model, f), dtype=np.float64)
+                     for f in ("eigenvalues", "col_sums", "rowsum_dots")]
+            if cnt.shape != (n_var,) or any(t.shape != (k,) for t in terms):
+                raise VpcaError(VPCA_ERR_BAD_ARG, "model: carriers must have V entries and the terms k")
+            vm = VpcaModel(ctypes.sizeof(VpcaModel), int(model.n_fitted), k, n_var, _host_ptr(L) if n_var else None,
+                           _host_ptr(cnt) if n_var else None, *[_host_ptr(t) for t in terms], float(model.matrix_mean))
+            rc = self._lib.vpca_create_scoring(ctypes.byref(cfg), ctypes.byref(vm), ctypes.byref(handle))
+            self.model_k = k
+        elif self.n_projected > 0 or sample_rows is not None:
             rows_map = None
             if sample_rows is not None:
                 rows_map = np.ascontiguousarray(sample_rows, dtype=np.int32)
@@ -589,6 +640,72 @@ class NativePca:
         flat = np.empty(max(self.n_projected * k, 1), dtype=np.float64)
         self._check(self._lib.vpca_project_pca(self._h, int(k), _host_ptr(flat)))
         return flat[:self.n_projected * k].reshape(k, self.n_projected).T.copy()
+
+    # -- saved model (DESIGN.md 3.7): loadings of a fitted context ... ----------------------------------------------
+    def pcaLoadingsCalls(self, k: int, offsets, sample_idx):
+        """Loadings of the rows of an accumulate call on the first k PCs of the last computePca: (L (nv, k) float64,
+        carriers (nv,) int32), one row per input variant."""
+        off, idx = self._csr(offsets, sample_idx)
+        nv = len(off) - 1
+        L, cnt = np.empty((nv, k), np.float64), np.empty(nv, np.int32)
+        self._check(self._lib.vpca_pca_loadings_calls(self._h, int(k), _host_ptr(off), _host_ptr(idx) if len(idx) else None,
+                                                      nv, _host_ptr(L), _host_ptr(cnt)))
+        return L, cnt
+
+    def pcaLoadingsBed(self, k: int, rows: np.ndarray, counted_allele: int = 1):
+        b = np.ascontiguousarray(rows, dtype=np.uint8)
+        if b.ndim != 2:
+            raise VpcaError(VPCA_ERR_BAD_ARG, "rows must be (nv, stride_bytes)")
+        L, cnt = np.empty((b.shape[0], k), np.float64), np.empty(b.shape[0], np.int32)
+        self._check(self._lib.vpca_pca_loadings_bed(self._h, int(k), _host_ptr(b), b.shape[0], b.shape[1],
+                                                    int(counted_allele), _host_ptr(L), _host_ptr(cnt)))
+        return L, cnt
+
+    def pcaLoadingsPanels(self, k: int, d_ptr: int, nv: int, panel_variants: int):
+        L, cnt = np.empty((nv, k), np.float64), np.empty(nv, np.int32)
+        self._check(self._lib.vpca_pca_loadings_panels(self._h, int(k), d_ptr, int(nv), int(panel_variants), _host_ptr(L),
+                                                       _host_ptr(cnt)))
+        return L, cnt
+
+    def pcaModelTerms(self, k: int) -> dict:
+        """eigenvalues, col_sums (a), rowsum_dots (b) and matrix_mean of the last computePca."""
+        ev, a, b = (np.empty(k, np.float64) for _ in range(3))
+        mm = np.empty(1, np.float64)
+        self._check(self._lib.vpca_pca_model_terms(self._h, int(k), _host_ptr(ev), _host_ptr(a), _host_ptr(b), _host_ptr(mm)))
+        return dict(eigenvalues=ev, col_sums=a, rowsum_dots=b, matrix_mean=float(mm[0]))
+
+    # -- ... and scoring of a study against it (contexts made with model=) -------------------------------------------
+    @staticmethod
+    def _model_rows(model_rows, nv: int) -> np.ndarray:
+        r = np.ascontiguousarray(model_rows, dtype=np.int32)
+        if r.shape != (nv,):
+            raise VpcaError(VPCA_ERR_BAD_ARG, f"model_rows must have one entry per variant ({nv})")
+        return r
+
+    def scoreCalls(self, partition_id: int, offsets, sample_idx, model_rows):
+        off, idx = self._csr(offsets, sample_idx)
+        r = self._model_rows(model_rows, len(off) - 1)
+        self._check(self._lib.vpca_score_calls(self._h, int(partition_id), _host_ptr(off), _host_ptr(idx) if len(idx) else None,
+                                               len(off) - 1, _host_ptr(r) if len(r) else None))
+
+    def scoreBed(self, partition_id: int, rows: np.ndarray, model_rows, counted_allele: int = 1):
+        b = np.ascontiguousarray(rows, dtype=np.uint8)
+        if b.ndim != 2:
+            raise VpcaError(VPCA_ERR_BAD_ARG, "rows must be (nv, stride_bytes)")
+        r = self._model_rows(model_rows, b.shape[0])
+        self._check(self._lib.vpca_score_bed(self._h, int(partition_id), _host_ptr(b), b.shape[0], b.shape[1],
+                                             int(counted_allele), _host_ptr(r) if len(r) else None))
+
+    def scorePanels(self, d_ptr: int, nv: int, panel_variants: int, model_rows):
+        r = self._model_rows(model_rows, nv)
+        self._check(self._lib.vpca_score_panels(self._h, d_ptr, int(nv), int(panel_variants), _host_ptr(r) if len(r) else None))
+
+    def scoreProject(self, k: int = 2):
+        """-> (y (n_samples, k) float64, matched variants): the study samples on the first k PCs of the model."""
+        flat = np.empty(self.n * k, dtype=np.float64)
+        matched = ctypes.c_int64(0)
+        self._check(self._lib.vpca_score_project(self._h, int(k), _host_ptr(flat), ctypes.byref(matched)))
+        return flat.reshape(k, self.n).T.copy(), int(matched.value)
 
     def getCentered(self) -> np.ndarray:
         out = np.empty((self.n, self.n), dtype=np.float64)

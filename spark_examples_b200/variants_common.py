@@ -29,6 +29,7 @@ class CallsBatch:
     """One partition already in `RDD[Seq[Int]]` form (VariantsPca.scala:153-168): CSR rows of sample indices."""
     offsets: np.ndarray   # int64, nv + 1
     idx: np.ndarray       # int32
+    keys: Optional[list] = None   # getVariantKey bytes of each row (kept for a saved model, model.py), else None
 
 
 @dataclass

@@ -25,6 +25,7 @@ from typing import Dict, Iterable, List, Optional, Sequence, Tuple
 import numpy as np
 
 from . import dist as vdist
+from . import model as vmodel
 from . import native
 from .conf import PcaConf
 from .jformat import jdouble
@@ -263,7 +264,9 @@ class VariantsPcaDriver:
                 if isinstance(part, (CallsBatch, SyntheticSlice, BedSlice, ParquetSlice)):
                     parts.append(part)                          # already RDD[Seq[Int]] rows (or their packed form)
                 else:
-                    parts.append(_rows_to_batch([extractCallInfo(v, mapping) for v in part]))
+                    # a saved model identifies the variants it keeps by their key (model.py)
+                    keys = [variantKeyBytes(v) for v in part] if self._model_flags() else None
+                    parts.append(_rows_to_batch([extractCallInfo(v, mapping) for v in part], keys))
             return CallsRdd(parts, n)
         # keying, join / merge and the concatenation of the calls run on the GPU and feed the encoder there (csrc/join.cu);
         # joinDatasets / mergeDatasets above stay as the record-level mirror of the reference's public methods
@@ -349,6 +352,104 @@ class VariantsPcaDriver:
         y = self._pca_nat.projectPca(self.conf.numPc())
         reverse, n = self._row_to_callset(), self.common.n_fitted
         return [(reverse[n + p], float(y[p, 0]), float(y[p, 1])) for p in range(self.common.n_projected)]
+
+    # -- saved model (model.py, DESIGN.md 3.7) ---------------------------------------------------------------------
+    def _model_flags(self) -> bool:
+        return self.conf.saveModel.isDefined or self.conf.modelPath.isDefined
+
+    def saveModel(self, callsets: CallsRdd) -> vmodel.PcaModel:
+        """After computePca: a second pass over the same partitions through the loadings route of each (calls / PLINK
+        rows / device panels), then the model file, written atomically.  Prints `Saved model: ...`."""
+        nat, k = self._pca_nat, self.conf.numPc()
+        vmodel.check_datasets(len(self.getData))
+        loadings, carriers, keys = [], [], []
+        source = vmodel.source_of(callsets.partitions) or "positional"
+        bim_keys = None
+        for part in callsets.partitions:
+            if isinstance(part, SyntheticSlice):
+                import torch
+                panel = 8192
+                buf = torch.empty(nat.panelBytes(part.nv, panel), dtype=torch.uint8, device=self._gram_tensor.device)
+                nat.synthPanelsDevice(part.seed, part.v0, part.nv, 0, buf.data_ptr(), panel)
+                L, c = nat.pcaLoadingsPanels(k, buf.data_ptr(), part.nv, panel)
+            elif isinstance(part, BedSlice):
+                if bim_keys is None:
+                    bim_keys = vmodel.plink_keys(part.bed.prefix)
+                L, c = nat.pcaLoadingsBed(k, part.rows(), part.counted)
+                keys.extend(bim_keys[part.v0:part.v0 + part.nv])
+            else:
+                if isinstance(part, ParquetSlice):
+                    part = part.load()
+                L, c = nat.pcaLoadingsCalls(k, part.offsets, part.idx)
+                if source == "records":
+                    keys.extend(part.keys)
+            loadings.append(L)
+            carriers.append(c)
+        terms = nat.pcaModelTerms(k)
+        counted = 0
+        if source == "plink":
+            counted = {"A1": 1, "A2": 2}[self.conf.bedCountedAllele().upper()]
+        m = vmodel.PcaModel(n_fitted=self.common.n_fitted, num_pc=k, loadings=np.concatenate(loadings) if loadings else
+                            np.zeros((0, k)), carriers=np.concatenate(carriers) if carriers else np.zeros(0, np.int32),
+                            keys=vmodel.hash_keys(nat, keys) if source != "positional" else np.zeros((0, 2), np.uint64),
+                            source=source, counted_allele=counted, max_multiplicity=nat.max_multiplicity, **terms)
+        vmodel.save(self.conf.saveModel(), m)
+        if self._rank == 0:
+            print(vmodel.saved_line(m))
+        return m
+
+    def scoreWithModel(self, callsets: CallsRdd) -> List[Tuple[str, float, float]]:
+        """Every callset of the input on the first two PCs of the saved model of --model-path: one pass over the
+        genotypes through the scoring route of each partition, no Gram and no eigensolve.  Prints the matched count."""
+        m = vmodel.load(self.conf.modelPath())
+        vmodel.check_datasets(len(self.getData))
+        k = self.conf.numPc()
+        if k < 2:
+            raise IndexError("the output reads the first two principal components; --num-pc must be >= 2")
+        source = vmodel.source_of(callsets.partitions) or "positional"
+        counted = {"A1": 1, "A2": 2}[self.conf.bedCountedAllele().upper()] if source == "plink" else 0
+        vmodel.check_study(m, k, source, counted, callsets.count())
+        n = len(self.common.indexes)
+        device = self.conf.gpuDevice() if self.conf.gpuDevice.isDefined else int(os.environ.get("LOCAL_RANK", "0"))
+        dtype = {"int8": native.DTYPE_I8, "i8": native.DTYPE_I8, "bf16": native.DTYPE_BF16}[self.conf.gpuDtype()]
+        nat = self._nat = native.NativePca(n, device=device, dtype=dtype, max_multiplicity=m.max_multiplicity, model=m)
+        index = vmodel.ModelIndex(m.keys) if m.keyed else None
+        bim_keys, v0 = None, 0
+        for pid, part in enumerate(callsets.partitions):
+            nv = part.nv if isinstance(part, (SyntheticSlice, BedSlice, ParquetSlice)) else len(part.offsets) - 1
+            if index is None:
+                rows = vmodel.positional_rows(v0, nv)
+            elif isinstance(part, BedSlice):
+                if bim_keys is None:
+                    bim_keys = vmodel.plink_keys(part.bed.prefix)
+                rows = index.rows(vmodel.hash_keys(nat, bim_keys[part.v0:part.v0 + part.nv]))
+            else:
+                rows = index.rows(vmodel.hash_keys(nat, part.keys))
+            v0 += nv
+            if isinstance(part, SyntheticSlice):
+                import torch
+                panel = 8192
+                buf = torch.empty(nat.panelBytes(part.nv, panel), dtype=torch.uint8, device=f"cuda:{device}")
+                nat.synthPanelsDevice(part.seed, part.v0, part.nv, 0, buf.data_ptr(), panel)
+                nat.scorePanels(buf.data_ptr(), part.nv, panel, rows)
+                nat.synchronize()                               # `buf` must outlive the kernels that read it
+                continue
+            try:
+                if isinstance(part, BedSlice):
+                    nat.scoreBed(pid, part.rows(), rows, part.counted)
+                else:
+                    if isinstance(part, ParquetSlice):
+                        part = part.load()
+                    nat.scoreCalls(pid, part.offsets, part.idx, rows)
+                nat.commit(pid)
+            except Exception:
+                nat.abort(pid)
+                raise
+        y, matched = nat.scoreProject(k)
+        if self._rank == 0:
+            print(vmodel.matched_line(matched, m))
+        reverse = {i: cid for cid, i in self.common.indexes.items()}
+        return [(reverse[i], float(y[i, 0]), float(y[i, 1])) for i in range(n)]
 
     def _row_to_callset(self) -> Dict[int, str]:
         rows = self.common.sample_rows
@@ -493,25 +594,37 @@ def joined_rows_on_host(p: JoinedSlice) -> CallsBatch:
     return CallsBatch(off, np.asarray([c for r in out for c in r], np.int32))
 
 
-def _rows_to_batch(rows: Iterable[Sequence[CallData]]) -> CallsBatch:
-    """VariantsPca.scala:164-167: keep calls with variation, drop empty variants, project to the callset index."""
-    kept = []
-    for calls in rows:
+def _rows_to_batch(rows: Iterable[Sequence[CallData]], keys: Optional[Sequence[bytes]] = None) -> CallsBatch:
+    """VariantsPca.scala:164-167: keep calls with variation, drop empty variants, project to the callset index.
+    keys (one per row): kept next to the rows that survive."""
+    kept, kept_keys = [], []
+    for v, calls in enumerate(rows):
         r = [c.callsetId for c in calls if c.hasVariation]
         if len(r) > 0:
             kept.append(r)
+            if keys is not None:
+                kept_keys.append(keys[v])
     off = np.zeros(len(kept) + 1, np.int64)
     if kept:
         off[1:] = np.cumsum([len(r) for r in kept])
         idx = np.concatenate([np.asarray(r, np.int32) for r in kept])
     else:
         idx = np.zeros(0, np.int32)
-    return CallsBatch(off, idx)
+    return CallsBatch(off, idx, kept_keys if keys is not None else None)
 
 
 def main(args: Optional[Sequence[str]] = None):
     """VariantsPcaDriver.main (VariantsPca.scala:38-50)."""
     conf = PcaConf(list(sys.argv[1:] if args is None else args))
+    vmodel.check_flags(conf, int(os.environ.get("WORLD_SIZE", "1")))
+    if conf.modelPath.isDefined:
+        driver = VariantsPcaDriver(conf)
+        vmodel.check_datasets(len(driver.getData))
+        callsRdd = driver.getCallsRdd([driver.filterDataset(d) for d in driver.getData])
+        driver.emitProjected(driver.scoreWithModel(callsRdd))
+        driver.reportIoStats()
+        driver.stop()
+        return
     if int(os.environ.get("WORLD_SIZE", "1")) > 1:
         import torch
         import torch.distributed as dist
@@ -519,6 +632,8 @@ def main(args: Optional[Sequence[str]] = None):
         dist.init_process_group("nccl")
     driver = VariantsPcaDriver(conf)
     data = driver.getData
+    if conf.saveModel.isDefined:
+        vmodel.check_datasets(len(data))
     filtered = [driver.filterDataset(d) for d in data]
     callsRdd = driver.getCallsRdd(filtered)
     simMatrix = driver.getSimilarityMatrix(callsRdd)
@@ -527,6 +642,8 @@ def main(args: Optional[Sequence[str]] = None):
     if conf.projectedCallsets.isDefined:
         driver.emitProjected(driver.projectPca())
     driver.reportIoStats()
+    if conf.saveModel.isDefined:
+        driver.saveModel(callsRdd)
     driver.stop()
     if int(os.environ.get("WORLD_SIZE", "1")) > 1:
         import torch.distributed as dist
